@@ -203,34 +203,40 @@ int ss4k_bsvd_stream_close(ss4k_bsvd_stream* s);
 /* image formats: 0 float NCHW, 1 half NCHW, 2 uint8 NHWC (read as value/255).  All pointers are DEVICE pointers. */
 /* per-(n,c) sum and sum of squares (double[n*c][2]); replaces .mean()/.std() of fsrcnn_upscaler.py:191-196,305-310 */
 int ss4k_glue_chan_stats(const void* img, int fmt, int n, int c, int h, int w, double* sums_dev, void* cuda_stream);
-/* F.interpolate(mode='area') -> float NCHW [n,c,oh,ow]  (fsrcnn_upscaler.py:174-176,204-209,239-241) */
+/* F.interpolate(mode='area') -> float NCHW [n,c,oh,ow]  (fsrcnn_upscaler.py:174-176,204-209,239-241);
+ * SS4K_E_INVALID unless n, c, h, w, oh, ow >= 1 */
 int ss4k_glue_area_pool(const void* img, int fmt, int n, int c, int h, int w, float* out_dev, int oh, int ow,
                         void* cuda_stream);
 /* low-res colour difference blur_k(a*hb + b - lb), reflect padding (fsrcnn_upscaler.py:211-213); a, b = the
- * distribution-match affine map derived from the sums (NULL sums: a=1, b=0) */
+ * distribution-match affine map derived from the sums (NULL sums: a=1, b=0).  SS4K_E_INVALID unless ksize is odd and
+ * positive, ksize/2 < h, ksize/2 < w (the limits of the reference's F.pad(mode='reflect')), n >= 1 and c >= 1 */
 int ss4k_glue_blur_diff(const float* hb, const float* lb, float* diff, const float* kern_dev, int ksize, int n, int c,
                         int h, int w, const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr,
                         void* cuda_stream);
 /* clamp(a*hr + b - bilinear_up(diff), 0, 1) -> uint8 NHWC (truncating unless round_u8) or float NCHW
- * (fsrcnn_upscaler.py:197-198,214-220,232-233); diff may be NULL */
+ * (fsrcnn_upscaler.py:197-198,214-220,232-233); diff may be NULL, otherwise dh >= 1 and dw >= 1 (SS4K_E_INVALID) */
 int ss4k_glue_finalize(const void* hr, int fmt, int n, int c, int h, int w, const float* diff, int dh, int dw,
                        const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* out_u8,
                        float* out_f32, int round_u8, void* cuda_stream);
 /* F.interpolate(mode='bicubic') of a float NCHW image, clamp, uint8 NHWC (fsrcnn_upscaler.py:222-233) */
 /* finalize + bicubic resize + uint8 in one pass (no full-resolution fp32 intermediate): the tail of upscale_multi /
- * upscale_single when output_shape differs from the net's output (fsrcnn_upscaler.py:214-233,315-326) */
+ * upscale_single when output_shape differs from the net's output (fsrcnn_upscaler.py:214-233,315-326).  c == 3;
+ * downscale factors up to about 2 (h/oh * 7 + 5 <= 24 and w/ow * 31 + 5 <= 72); diff NULL or dh, dw >= 1 */
 int ss4k_glue_finalize_bicubic_u8(const void* hr, int fmt, int n, int c, int h, int w, const float* diff, int dh, int dw,
                                   const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr,
                                   uint8_t* out_u8, int oh, int ow, int round_u8, void* cuda_stream);
+/* SS4K_E_INVALID unless n, c, h, w, oh, ow >= 1 */
 int ss4k_glue_bicubic_u8(const float* in, int n, int c, int h, int w, uint8_t* out, int oh, int ow, int round_u8,
                          void* cuda_stream);
 /* opacity * clamp(sharpen_ker(strength)(x), 0, 1) + (1-opacity) * other -> float NCHW; other may be NULL
- * (fsrcnn_upscaler.py:54-84,278-281,298-299) */
+ * (fsrcnn_upscaler.py:54-84,278-281,298-299).  SS4K_E_INVALID for h < 2 or w < 2 (3x3 reflect padding) */
 int ss4k_glue_sharpen_blend(const void* x, int fmt, int n, int c, int h, int w, float strength, float opacity,
                             const void* other, int other_fmt, float* out, void* cuda_stream);
 /* the same, written as an upscaler plan's first-layer activation tensor (ss4k_plan_input_act: 16-bit NHWC, channel
  * pitch `pitch`, pixel_unshuffle(`unshuffle`) channel order): the denoise -> upscale hand-over of upscale_single
- * (fsrcnn_upscaler.py:278-295) without a float image and without a layout kernel in front of conv_first */
+ * (fsrcnn_upscaler.py:278-295) without a float image and without a layout kernel in front of conv_first.
+ * SS4K_E_INVALID for h < 2 or w < 2, h or w not a multiple of unshuffle, pitch not a multiple of 8 or below
+ * c * unshuffle^2 */
 int ss4k_glue_sharpen_blend_act(const void* x, int fmt, int n, int c, int h, int w, float strength, float opacity,
                                 const void* other, int other_fmt, void* act_out, int unshuffle, int pitch, int is_bf16,
                                 void* cuda_stream);

@@ -612,7 +612,7 @@ int ss4k_glue_chan_stats(const void* img, int fmt, int n, int c, int h, int w, d
 }
 
 int ss4k_glue_area_pool(const void* img, int fmt, int n, int c, int h, int w, float* out_dev, int oh, int ow, void* stream) {
-  if (!img || !out_dev || fmt < 0 || fmt > 2 || oh < 1 || ow < 1) return SS4K_E_INVALID;
+  if (!img || !out_dev || fmt < 0 || fmt > 2 || n < 1 || c < 1 || h < 1 || w < 1 || oh < 1 || ow < 1) return SS4K_E_INVALID;
   const size_t total = static_cast<size_t>(n) * c * oh * ow;
   area_pool_kernel<<<blocks_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(Img{img, fmt, n, c, h, w}, out_dev, oh, ow);
   return cudaGetLastError() == cudaSuccess ? SS4K_OK : SS4K_E_CUDA;
@@ -620,7 +620,9 @@ int ss4k_glue_area_pool(const void* img, int fmt, int n, int c, int h, int w, fl
 
 int ss4k_glue_blur_diff(const float* hb, const float* lb, float* diff, const float* kern_dev, int ksize, int n, int c, int h,
                         int w, const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr, void* stream) {
-  if (!hb || !lb || !diff || !kern_dev) return SS4K_E_INVALID;
+  if (!hb || !lb || !diff || !kern_dev || n < 1 || c < 1) return SS4K_E_INVALID;
+  // reflect() mirrors an index once: the radius must stay below both sizes (F.pad(mode='reflect') refuses the rest)
+  if (ksize < 1 || ksize % 2 == 0 || ksize / 2 >= h || ksize / 2 >= w) return SS4K_E_INVALID;
   const size_t total = static_cast<size_t>(n) * c * h * w;
   blur_diff_kernel<<<blocks_for(total, 128), 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(hb, lb, diff, kern_dev, ksize, n, c, h, w,
                                                                                            hr_sums, lr_sums, cnt_hr, cnt_lr);
@@ -631,6 +633,7 @@ int ss4k_glue_finalize(const void* hr, int fmt, int n, int c, int h, int w, cons
                        const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* out_u8,
                        float* out_f32, int round_u8, void* stream) {
   if (!hr || (!out_u8 && !out_f32) || fmt < 0 || fmt > 1) return SS4K_E_INVALID;
+  if (diff && (dh < 1 || dw < 1)) return SS4K_E_INVALID;
   const size_t total = static_cast<size_t>(n) * h * w;
   finalize_kernel<<<blocks_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(Img{hr, fmt, n, c, h, w}, diff, dh, dw, hr_sums,
                                                                                           lr_sums, cnt_hr, cnt_lr, out_u8, out_f32, round_u8);
@@ -641,6 +644,7 @@ int ss4k_glue_finalize_bicubic_u8(const void* hr, int fmt, int n, int c, int h, 
                                   const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* out_u8,
                                   int oh, int ow, int round_u8, void* stream) {
   if (!hr || !out_u8 || fmt < 0 || fmt > 1 || c != 3 || oh <= 0 || ow <= 0) return SS4K_E_INVALID;
+  if (diff && (dh < 1 || dw < 1)) return SS4K_E_INVALID;
   // the tile kernel's shared-memory patch covers downscale factors up to 2 (plus the 3-pixel tap margin)
   const double fy = static_cast<double>(h) / oh, fx = static_cast<double>(w) / ow;
   if (fy * (kFbTh - 1) + 5.0 > kFbMaxH || fx * (kFbTw - 1) + 5.0 > kFbMaxW) return SS4K_E_INVALID;
@@ -651,7 +655,7 @@ int ss4k_glue_finalize_bicubic_u8(const void* hr, int fmt, int n, int c, int h, 
 }
 
 int ss4k_glue_bicubic_u8(const float* in, int n, int c, int h, int w, uint8_t* out, int oh, int ow, int round_u8, void* stream) {
-  if (!in || !out) return SS4K_E_INVALID;
+  if (!in || !out || n < 1 || c < 1 || h < 1 || w < 1 || oh < 1 || ow < 1) return SS4K_E_INVALID;
   const size_t total = static_cast<size_t>(n) * oh * ow;
   bicubic_u8_kernel<<<blocks_for(total, 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(in, n, c, h, w, out, oh, ow, round_u8);
   return cudaGetLastError() == cudaSuccess ? SS4K_OK : SS4K_E_CUDA;
@@ -660,6 +664,7 @@ int ss4k_glue_bicubic_u8(const float* in, int n, int c, int h, int w, uint8_t* o
 int ss4k_glue_sharpen_blend(const void* x, int fmt, int n, int c, int h, int w, float strength, float opacity, const void* other,
                             int other_fmt, float* out, void* stream) {
   if (!x || !out || fmt < 0 || fmt > 2 || (other && (other_fmt < 0 || other_fmt > 3))) return SS4K_E_INVALID;
+  if (h < 2 || w < 2) return SS4K_E_INVALID;  // the 3x3 reflect needs a neighbour on each side
   // sharpen_ker (fsrcnn_upscaler.py:54-84): (sharp*s + identity*(1-s)) / sum, sharp = [-1..9..-1]
   const float center = 9.f * strength + (1.f - strength), side = -strength;
   const float sum = center + 8.f * side;
@@ -675,6 +680,7 @@ int ss4k_glue_sharpen_blend(const void* x, int fmt, int n, int c, int h, int w, 
 int ss4k_glue_sharpen_blend_act(const void* x, int fmt, int n, int c, int h, int w, float strength, float opacity, const void* other,
                                 int other_fmt, void* act_out, int unshuffle, int pitch, int bf16, void* stream) {
   if (!x || !act_out || fmt < 0 || fmt > 2 || (other && (other_fmt < 0 || other_fmt > 3))) return SS4K_E_INVALID;
+  if (h < 2 || w < 2) return SS4K_E_INVALID;
   if (unshuffle < 1 || h % unshuffle || w % unshuffle || pitch % 8 || pitch < c * unshuffle * unshuffle) return SS4K_E_INVALID;
   const float center = 9.f * strength + (1.f - strength), side = -strength;
   const float sum = center + 8.f * side;

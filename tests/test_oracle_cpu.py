@@ -117,6 +117,9 @@ def test_glue_kernels_match_reference_formulas():
     assert abs(k.sum().item() - 1.0) < 1e-6 and abs(k[0, 0, 1, 1].item() - (1 + 8 * 0.00002)) < 1e-6
     b = glue.blur_weight(17, 8.0)
     assert abs(b.sum().item() - 1.0) < 1e-5 and b[0, 0, 8, 8] == b.max()
+    # the service's colour-match blur weights (service.py: gaussian_kernel(17, 8.0)) are blur_ker's
+    from ss4k_b200 import service
+    assert (service.gaussian_kernel(17, 8.0).double() - b[0, 0].double()).abs().max().item() <= 1e-9
     frames = torch.randint(0, 256, (2, 24, 32, 3), dtype=torch.uint8)
     up = lambda t: torch.nn.functional.interpolate(t, scale_factor=2, mode="bicubic")  # noqa: E731
     out = glue.upscale_multi(frames, up, lr_shape=(24, 32), output_shape=(48, 64))
