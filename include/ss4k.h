@@ -87,7 +87,14 @@ typedef struct ss4k_plan_cfg {
   int32_t tile_pad;
   int32_t act_mode;    /* SS4K_ACT_*                                          */
   int32_t in_fmt;      /* SS4K_FMT_*                                          */
-  int32_t out_fmt;     /* SS4K_FMT_* (U8: clamp to [0,1], *255, truncate like fsrcnn_upscaler.py:233) */
+  int32_t out_fmt;     /* SS4K_FMT_* (U8: clamp to [0,1], *255, truncate like fsrcnn_upscaler.py:233).
+                        * NV12 (SS4K_ARCH_RRDB only; SRVGG and BSVD plans return SS4K_E_INVALID): packed frames
+                        * [n, oh*3/2, ow] bytes, the Y plane u8[oh,ow] then interleaved UV u8[oh/2,ow] per frame (the layout
+                        * in_fmt SS4K_FMT_NV12 and ss4k_nv12_unpack use); oh % 2 == 0 and ow % 4 == 0 are required.  The
+                        * result is bit-identical to ss4k_rgb_to_nv12 applied to the same plan's SS4K_FMT_U8_NHWC output.
+                        * Untiled plans convert in the last convolution's epilogue; tiled plans (and a last convolution
+                        * off the streaming kernel) write uint8 RGB into a frame of the plan and convert it in a step of
+                        * its own. */
   int32_t use_graph;   /* 1: capture the per-frame launch sequence in a CUDA graph */
   int32_t reserved[8]; /* [1]: RealESRGANer pre_pad (factory.py:95): reflect pad on the right / bottom before tiling, cropped
                         *      off the output; the x2 nets also get RealESRGANer's reflect mod-2 pad for odd sizes.  tile,
@@ -119,7 +126,8 @@ int ss4k_clear_weights(ss4k_ctx* ctx, int net_id);
 /* plans -------------------------------------------------------------------------------- */
 int ss4k_plan_create(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_plan);
 int ss4k_plan_destroy(ss4k_plan* plan);
-/* output geometry of a plan: n, c, h, w of the result tensor */
+/* output geometry of a plan: n, c, h, w of the result image (NV12 output: still (n, 3, oh, ow); the buffer holds
+ * n * oh * ow * 3 / 2 bytes, as ss4k_plan_io_bytes reports) */
 int ss4k_plan_out_shape(const ss4k_plan* plan, int32_t out_nchw[4]);
 /* algorithmic FLOPs of one ss4k_run (2*Cin*Cout*9*Hout*Wout summed over convs, true channel counts) */
 double ss4k_plan_flops(const ss4k_plan* plan);
@@ -151,11 +159,15 @@ int ss4k_run_host(ss4k_plan* plan, const void* in_host, void* out_host);
  * out_host buffers are in flight, so alternate between two. */
 int ss4k_run_host_async(ss4k_plan* plan, const void* in_host, void* out_host);
 int ss4k_plan_host_sync(ss4k_plan* plan);
+/* bytes of one run's input / output buffer in the plan's in_fmt / out_fmt (NV12: n * h * w * 3 / 2); ss4k_run_host and
+ * ss4k_run_host_async copy exactly these sizes */
 int ss4k_plan_io_bytes(const ss4k_plan* plan, int64_t* in_bytes, int64_t* out_bytes);
 /* measurement entry (bench.py roofline): one run of the plan without its CUDA graph, a CUDA event between
  * every step on `cuda_stream`.  ms[i] = device time of step i, flops[i] = its algorithmic FLOPs,
- * kind[i] = 0 layout/colour kernel, 1 row-streaming conv kernel, 2 tile conv kernel.  Returns the step
- * count (<= cap) or a negative error. */
+ * kind[i] = 0 layout/colour kernel, 1 row-streaming conv kernel, 2 tile conv kernel, 3 fused residual dense block,
+ * 4 a conv inside the fused launch in front of it.  An NV12-output plan whose last conv does not store NV12 itself has
+ * one more step at the end: the uint8 RGB -> NV12 conversion (kind 0).  Returns the step count (<= cap) or a negative
+ * error. */
 int ss4k_plan_profile(ss4k_plan* plan, const void* in_dev, void* out_dev, void* cuda_stream, float* ms,
                       double* flops, int32_t* kind, int cap);
 

@@ -32,7 +32,9 @@ enum OutMode : int {
   kOutScatterNHWC = 4,// BSVD temporal shift: channel slices go to the t-1 / t+1 / t ring slots
   kOutNCHWF16 = 5,
   kOutU8NHWC = 6,     // clamp [0,1], *255, truncate or round, uint8 NHWC (3 channels)
-  kOutPSNCHWF16 = 7   // like kOutPSNCHWF32 with a half-precision destination
+  kOutPSNCHWF16 = 7,  // like kOutPSNCHWF32 with a half-precision destination
+  kOutNV12 = 8        // the kOutU8NHWC bytes converted to NV12 (Y plane + interleaved UV per frame, BT.709 limited range,
+                      // rgb_to_nv12_kernel's arithmetic): streaming kernel, NOUT == 16, cout == 3 only (conv_stream.cu)
 };
 
 enum ActKind : int { kActNone = 0, kActPRelu = 1, kActRelu6 = 2 };
@@ -135,6 +137,11 @@ constexpr int kStreamOnesBytes = 128 * 128;  // "ones" operand tile of the bias 
 
 constexpr int kStreamEpiWarps = 8;  // two per TMEM lane quarter, alternating output rows
 constexpr int kStreamThreads = 32 * (2 + kStreamEpiWarps);
+// kOutNV12: chroma hand-over between the two epilogue warps of a lane quarter -- one named barrier per quarter (IDs
+// kNv12BarBase .. +3; ID 1 is the set-up barrier) and 2 slots x 4 quarters x 16 pixel pairs of packed 32-bit sums in
+// shared memory behind the row records
+constexpr int kNv12BarBase = 2;
+constexpr int kNv12XchgBytes = 2 * 4 * 16 * 4;
 constexpr int kMaskRects = 16;                 // crops per atlas image
 constexpr int kMaskStride = 1 + 3 * kMaskRects;  // int32 words per image in StreamParams::mask_hw
 constexpr int kStreamSrcWarps = 2;  // frame-format source (StreamParams::src_fmt): decoder warps on top, alternating input rows

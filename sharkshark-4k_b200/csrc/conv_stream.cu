@@ -265,8 +265,12 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
     for (int i = 0; i < static_cast<int>(sizeof(StreamParams) / 64); ++i) acc ^= pw[i * 8];
     asm volatile("" ::"l"(acc));
   }
-  const int u0 = static_cast<int>(static_cast<int64_t>(blockIdx.x) * P.total_units / gridDim.x);
-  const int u1 = static_cast<int>(static_cast<int64_t>(blockIdx.x + 1) * P.total_units / gridDim.x);
+  // NV12 store: rows are split in pairs, so that both rows of a chroma row pair belong to one CTA and (H even) every
+  // band starts on an even row: the row counter's parity is the row's parity, row 2j goes to the parity-0 warp and row
+  // 2j+1 to the parity-1 warp of the same lane quarter
+  const int pair_sh = (NOUT == 16 && P.ep.out_mode == kOutNV12) ? 1 : 0;
+  const int u0 = static_cast<int>(static_cast<int64_t>(blockIdx.x) * (P.total_units >> pair_sh) / gridDim.x) << pair_sh;
+  const int u1 = static_cast<int>(static_cast<int64_t>(blockIdx.x + 1) * (P.total_units >> pair_sh) / gridDim.x) << pair_sh;
   int early_chunk = -1;  // weights requested in the prologue (producer warp)
   if (warp == 0) {
     // barrier set-up spread over the warp's lanes (58 dependent shared-memory operations from one lane were a
@@ -1068,6 +1072,50 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                   if (split_store) tma_store_4d(&P.tmO2, stage + kStageWarp, b.chunk * NOUT, b.strip * kTileW + qd * 32, y, b.n + P.n_out0, pol_out);
                 }
                 bulk_commit();
+              }
+            } else if (NOUT == 16 && E.out_mode == kOutNV12) {
+              if constexpr (NOUT == 16) {
+                // NV12 frame store (RRDBNet's conv_last, out_fmt SS4K_FMT_NV12): the bytes of the kOutU8NHWC path, converted
+                // with rgb_to_nv12_kernel's integer arithmetic (elementwise.cu).  Each warp stores its own Y row; the
+                // parity-0 warp (row 2j) leaves its horizontal chroma pair sums in shared memory, the parity-1 warp (row
+                // 2j+1) adds its own and stores UV row j.  Both warps take the quarter's named barrier once per row pair
+                // whatever their `valid` lanes.  Two exchange slots suffice: the parity-0 warp refills slot j & 1 only
+                // after the barrier of pair j+1, which the parity-1 warp reaches after it has read pair j's sums.
+                // (W % 4 == 0 and strips start at multiples of 128: a 4-pixel word is entirely valid or entirely not.)
+                int c8[3];
+#pragma unroll
+                for (int i = 0; i < 3; ++i) {
+                  float f = fminf(fmaxf(__uint_as_float(raw[i]), 0.f), 1.f) * 255.f;
+                  if (E.round_u8) f = rintf(f);
+                  c8[i] = static_cast<uint8_t>(f);
+                }
+                const uint32_t yv = static_cast<uint32_t>(16 + ((5983 * c8[0] + 20127 * c8[1] + 2032 * c8[2] + 16384) >> 15));
+                uint32_t yw = yv | (__shfl_down_sync(0xffffffffu, yv, 1) << 8);
+                yw |= __shfl_down_sync(0xffffffffu, yw, 2) << 16;   // lane 4i: Y of pixels 4i .. 4i+3
+                // R, G, B of the pixel pair (lanes 2i, 2i+1) as 10-bit fields: a 2x2 sum is at most 1020
+                const uint32_t hs1 = static_cast<uint32_t>(c8[0]) | (static_cast<uint32_t>(c8[1]) << 10) | (static_cast<uint32_t>(c8[2]) << 20);
+                const uint32_t hs = hs1 + __shfl_xor_sync(0xffffffffu, hs1, 1);
+                uint8_t* const frame = reinterpret_cast<uint8_t*>(E.out) + static_cast<size_t>(b.n) * (E.out_h + (E.out_h >> 1)) * E.out_w;
+                const bool st_word = valid && (lane & 3) == 0;
+                if (st_word) *reinterpret_cast<uint32_t*>(frame + static_cast<size_t>(y) * E.out_w + ax) = yw;
+                const uint32_t xchg = rec_base + kMaxSASlots * kRecWords * 4u +
+                                      ((((static_cast<uint32_t>(q) >> 1) & 1u) * 4u + static_cast<uint32_t>(qd)) * 16u + (lane >> 1)) * 4u;
+                if (par == 0 && (lane & 1) == 0) asm volatile("st.shared.b32 [%0], %1;" ::"r"(xchg), "r"(hs) : "memory");
+                asm volatile("bar.sync %0, 64;" ::"r"(kNv12BarBase + qd) : "memory");
+                if (par == 1) {
+                  uint32_t s4 = hs;
+                  if ((lane & 1) == 0) {
+                    uint32_t other;
+                    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(other) : "r"(xchg) : "memory");
+                    s4 += other;
+                  }
+                  const int sr = static_cast<int>(s4 & 0x3FFu), sg = static_cast<int>((s4 >> 10) & 0x3FFu), sb = static_cast<int>(s4 >> 20);
+                  const int uu = 128 + ((-3298 * sr - 11094 * sg + 14392 * sb + 65536) >> 17);
+                  const int vv = 128 + ((14392 * sr - 13073 * sg - 1319 * sb + 65536) >> 17);
+                  uint32_t uvw = (static_cast<uint32_t>(uu) & 0xFFu) | ((static_cast<uint32_t>(vv) & 0xFFu) << 8);
+                  uvw |= __shfl_down_sync(0xffffffffu, uvw, 2) << 16;   // lane 4i: U, V of pairs 2i, 2i+1
+                  if (st_word) *reinterpret_cast<uint32_t*>(frame + static_cast<size_t>(E.out_h + (y >> 1)) * E.out_w + ax) = uvw;
+                }
               }
             } else if (NOUT == 16 && E.out_mode == kOutU8NHWC && E.cout == 3 && E.act == kActNone && E.alpha == 1.0f &&
                        E.res1 == nullptr && E.res2 == nullptr && __all_sync(0xffffffffu, valid)) {

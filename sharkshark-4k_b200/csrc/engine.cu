@@ -398,6 +398,14 @@ bool stream_config(const ConvSpec& cs, StreamPacked* sp) {
   return false;
 }
 
+// kOutNV12 is stored by the <16> streaming kernel's epilogue (conv_stream.cu); a conv that runs elsewhere writes uint8 RGB
+// and the plan converts it (ss4k_plan_create)
+bool stream_nv12_ok(const ConvSpec& cs) {
+  StreamPacked sp;
+  return stream_config(cs, &sp) && sp.nout == 16 && sp.chunks == 1 && cs.cout == 3 && cs.act == kActNone && cs.alpha == 1.f &&
+         cs.res1_buf < 0 && cs.res2_buf < 0 && cs.out_h % 2 == 0 && cs.out_w % 4 == 0;
+}
+
 std::string pack_weights_stream(const ConvSpec& cs, const HostTensor& W, const HostTensor* B, const HostTensor* S,
                                 bool bf16, StreamPacked* out) {
   if (W.shape.size() != 4 || W.shape[0] != cs.cout || W.shape[1] != cs.cin || W.shape[2] != 3 || W.shape[3] != 3)
@@ -889,6 +897,10 @@ struct ss4k_plan {
   int n_fused = 0;
   void* stage_in = nullptr;   // device staging for ss4k_run_host
   void* stage_out = nullptr;
+  // NV12 output in two steps (tiled plans, or a last conv that does not run on the streaming kernel): the uint8 RGB frame
+  // the last conv / the tile paste writes, converted into the caller's buffer by the rgb_to_nv12 kernel.  Null when the
+  // last conv's epilogue stores NV12 itself.
+  void* nv12_rgb = nullptr;
   // software pipeline of ss4k_run_host_async: two staging slots, copy streams, hand-over events
   struct HostPipe {
     void* in[2] = {nullptr, nullptr};
@@ -939,11 +951,16 @@ int run_step(ss4k_plan* pl, int si, const void* in_dev, void* out_dev, cudaStrea
                         p.out_lo_buf >= 0 ? reinterpret_cast<uint8_t*>(pl->bufs[p.out_lo_buf]) + out_off : nullptr,
                         p.n, p.c, p.h, p.w, ob.pitch, p.unshuffle, p.fill_ch, p.fill_val, bf16 ? 1 : 0, st));
     ctx->launches++;
+  } else if (s.kind == 2) {
+    const Program& P = pl->prog;
+    CK(ctx, rgb_to_nv12_launch(pl->nv12_rgb, out_dev, P.out_n, P.out_h, P.out_w, st));
+    ctx->launches++;
   } else {
     ConvExec& c = pl->convs[pl->step_conv[si]];
     if (c.skip) return SS4K_OK;
     if (c.src_ext) c.sp.src = reinterpret_cast<const uint8_t*>(in_dev) + c.src_off;
-    CK(ctx, launch_exec(c, out_dev, st));
+    // (two-step NV12 output: the last conv writes the plan's uint8 RGB frame, the conversion step the caller's buffer)
+    CK(ctx, launch_exec(c, c.ext_out && pl->nv12_rgb != nullptr ? pl->nv12_rgb : out_dev, st));
     ctx->launches++;
   }
   return SS4K_OK;
@@ -1105,7 +1122,7 @@ int fuse_rdbs(ss4k_plan* pl) {
 }
 
 bool step_is_external(const Step& s) {
-  if (s.kind == 0) return true;  // prep reads the caller's pointer
+  if (s.kind != 1) return true;  // prep reads the caller's pointer, the NV12 conversion writes it
   return s.conv.out_buf == kBufExternalOut;
 }
 
@@ -1297,6 +1314,7 @@ int ss4k_plan_destroy(ss4k_plan* pl) {
   }
   if (pl->stage_in) cudaFree(pl->stage_in);
   if (pl->stage_out) cudaFree(pl->stage_out);
+  if (pl->nv12_rgb) cudaFree(pl->nv12_rgb);
   if (pl->d_ctr) cudaFree(pl->d_ctr);
   if (pl->d_rdb_trace) cudaFree(pl->d_rdb_trace);
   if (pl->d_mask) cudaFree(pl->d_mask);
@@ -1342,8 +1360,13 @@ int ss4k_plan_create(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_pl
   // convs
   pl->step_conv.assign(P.steps.size(), -1);
   pl->convs.reserve(P.steps.size());
+  bool nv12_two_step = false;
   for (size_t si = 0; si < P.steps.size(); ++si) {
     if (P.steps[si].kind != 1) continue;
+    if (P.steps[si].conv.out_mode == kOutNV12 && !stream_nv12_ok(P.steps[si].conv)) {
+      P.steps[si].conv.out_mode = kOutU8NHWC;   // two-step form: uint8 RGB into pl->nv12_rgb, then the conversion step
+      nv12_two_step = true;
+    }
     const ConvSpec& cs = P.steps[si].conv;
     auto w = wmap.find(cs.wname);
     if (w == wmap.end()) { int rc = fail(ctx, SS4K_E_WEIGHTS, "missing weight " + cs.wname); ss4k_plan_destroy(pl.release()); return rc; }
@@ -1363,6 +1386,14 @@ int ss4k_plan_create(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_pl
     pl->step_conv[si] = static_cast<int>(pl->convs.size()) - 1;
     int rc = materialize_conv(ctx, cs, w->second, B, S, cfg->act_mode, bufptr, &pl->convs.back());
     if (rc != SS4K_OK) { ss4k_plan_destroy(pl.release()); return rc; }
+  }
+  if (nv12_two_step) {
+    cudaError_t ce = cudaMalloc(&pl->nv12_rgb, fmt_bytes(SS4K_FMT_U8_NHWC, P.out_n, 3, P.out_h, P.out_w) + 256);
+    if (ce != cudaSuccess) { ss4k_plan_destroy(pl.release()); return fail(ctx, SS4K_E_NOMEM, "NV12 output: uint8 RGB frame"); }
+    Step s;
+    s.kind = 2;
+    P.steps.push_back(s);
+    pl->step_conv.push_back(-1);
   }
   {
     int rc = fuse_rdbs(pl.get());
@@ -1562,10 +1593,14 @@ static std::string layout_tiles(const ss4k_plan_cfg* cfg, std::vector<TileGroup>
 static int create_tiled_plan(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_plan) {
   std::vector<TileGroup> groups;
   {
-    const std::string e = layout_tiles(cfg, &groups);
+    std::string e = nv12_out_check(lite(cfg));
+    if (e.empty()) e = layout_tiles(cfg, &groups);
     if (!e.empty()) return fail(ctx, SS4K_E_INVALID, e);
   }
   const int s = cfg->scale;
+  // NV12 output: the tile classes paste uint8 RGB into a frame of the plan, converted once per run (crops need not have
+  // NV12-compatible sizes)
+  const bool nv12 = cfg->out_fmt == SS4K_FMT_NV12;
   std::unique_ptr<ss4k_plan> pl(new ss4k_plan());
   pl->ctx = ctx;
   pl->cfg = *cfg;
@@ -1582,6 +1617,7 @@ static int create_tiled_plan(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan*
     uniform = uniform && g.nimg == tc.count;
     ss4k_plan_cfg sub = *cfg;
     sub.tile = 0; sub.reserved[1] = 0;
+    if (nv12) sub.out_fmt = SS4K_FMT_U8_NHWC;
     sub.reserved[5] = uniform ? 0 : 1;
     sub.n = cfg->n * tc.nimg; sub.h = tc.hc; sub.w = tc.wc;
     pl->tiles.push_back(tc);
@@ -1618,6 +1654,10 @@ static int create_tiled_plan(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan*
   }
   pl->in_bytes = fmt_bytes(P.in_fmt, P.in_n, P.in_c, P.in_h, P.in_w);
   pl->out_bytes = fmt_bytes(P.out_fmt, P.out_n, P.out_c, P.out_h, P.out_w);
+  if (nv12 && cudaMalloc(&pl->nv12_rgb, fmt_bytes(SS4K_FMT_U8_NHWC, P.out_n, 3, P.out_h, P.out_w) + 256) != cudaSuccess) {
+    ss4k_plan_destroy(pl.release());
+    return fail(ctx, SS4K_E_NOMEM, "NV12 output: uint8 RGB frame");
+  }
   cudaDeviceSynchronize();   // the tile boxes were uploaded on the NULL stream
   *out_plan = pl.release();
   return SS4K_OK;
@@ -1701,6 +1741,7 @@ int ss4k_plan_launches(const ss4k_plan* pl) {
   if (!pl) return 0;
   int n = live_steps(pl, 0, static_cast<int>(pl->prog.steps.size()) - 1);
   for (const auto& t : pl->tiles) n += ss4k_plan_launches(t.sub) + 2;   // + gather and paste of the tile class
+  if (pl->tiled && pl->nv12_rgb != nullptr) n += 1;                      // + the NV12 conversion of the pasted frame
   return n;
 }
 int ss4k_plan_graph_steps(const ss4k_plan* pl) {
@@ -1734,13 +1775,18 @@ int ss4k_run(ss4k_plan* pl, const void* in_dev, void* out_dev, void* cuda_stream
   cudaStream_t st = reinterpret_cast<cudaStream_t>(cuda_stream);
   if (pl->tiled) {
     const Program& P = pl->prog;
+    const bool nv12 = pl->nv12_rgb != nullptr;   // paste uint8 RGB into the plan's frame, convert it at the end
     for (auto& t : pl->tiles) {
       CK(ctx, tile_gather_launch(P.in_fmt, in_dev, t.d_in, t.d_boxes, t.count, t.nimg, P.in_n, 3, P.in_h, P.in_w, pl->cfg.reserved[1], t.hc, t.wc, st));
       int rc = ss4k_run(t.sub, t.d_in, t.d_out, cuda_stream);
       if (rc != SS4K_OK) return rc;
-      CK(ctx, tile_paste_launch(P.out_fmt, t.d_out, out_dev, t.d_boxes, t.count, P.in_n, 3, t.sub->prog.out_h, t.sub->prog.out_w,
-                                pl->cfg.scale, P.out_h, P.out_w, st));
+      CK(ctx, tile_paste_launch(nv12 ? SS4K_FMT_U8_NHWC : P.out_fmt, t.d_out, nv12 ? pl->nv12_rgb : out_dev, t.d_boxes, t.count, P.in_n, 3,
+                                t.sub->prog.out_h, t.sub->prog.out_w, pl->cfg.scale, P.out_h, P.out_w, st));
       ctx->launches += 2;
+    }
+    if (nv12) {
+      CK(ctx, rgb_to_nv12_launch(pl->nv12_rgb, out_dev, P.out_n, P.out_h, P.out_w, st));
+      ctx->launches += 1;
     }
     return SS4K_OK;
   }
@@ -1883,6 +1929,7 @@ int ss4k_plan_profile(ss4k_plan* pl, const void* in_dev, void* out_dev, void* cu
     cudaEventElapsedTime(&ms[si], ev[si], ev[si + 1]);
     const Step& s = pl->prog.steps[si];
     flops[si] = s.kind == 1 ? s.conv.flops() : 0.0;
+    if (s.kind == 2) { kind[si] = 0; continue; }   // the NV12 conversion of a two-step NV12 output: a colour kernel
     kind[si] = s.kind == 0 ? (si == pl->fused_prep ? 4 : 0) : (pl->convs[pl->step_conv[si]].stream ? 1 : 2);
     if (s.kind == 1) {
       const ConvExec& c = pl->convs[pl->step_conv[si]];

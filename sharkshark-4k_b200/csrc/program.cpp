@@ -30,6 +30,7 @@ int final_out_mode(int out_fmt) {
     case 0: return kOutNCHWF32;
     case 1: return kOutNCHWF16;
     case 2: return kOutU8NHWC;
+    case 3: return kOutNV12;
     default: return -1;
   }
 }
@@ -38,7 +39,7 @@ int final_out_mode(int out_fmt) {
 std::string build_srvgg(const PlanCfgLite& c, Program* P) {
   const int s = c.scale;
   if (s != 2 && s != 4 && s != 1 && s != 3) return "SRVGG: unsupported upscale";
-  if (c.out_fmt != 0 && c.out_fmt != 1) return "SRVGG: output is float / half NCHW";
+  if (c.out_fmt != 0 && c.out_fmt != 1) return "SRVGG: output is float / half NCHW (the colour-match glue reads it; no uint8 / NV12 output)";
   const int nf = 64, nconv = c.depth > 0 ? c.depth : 16;
   const int cl = 3 * s * s;
   P->in_n = c.n; P->in_c = 3; P->in_h = c.h; P->in_w = c.w;
@@ -90,6 +91,7 @@ std::string build_rrdb(const PlanCfgLite& c, Program* P) {
   const int us = (s == 2) ? 2 : 1;
   if (c.h % us || c.w % us) return "RRDBNet x2: H and W must be even (mod_scale, RealESRGANer.pre_process)";
   const int th = c.h / us, tw = c.w / us;  // trunk resolution
+  if (c.out_fmt == 3 && ((th * 4) % 2 || (tw * 4) % 4)) return "RRDBNet: NV12 output needs an even height and a width divisible by 4";
   const int cin0 = 3 * us * us;
   P->in_n = c.n; P->in_c = 3; P->in_h = c.h; P->in_w = c.w;
   P->out_n = c.n; P->out_c = 3; P->out_h = th * 4; P->out_w = tw * 4;
@@ -189,6 +191,8 @@ std::string build_rrdb(const PlanCfgLite& c, Program* P) {
     v.act = kActPRelu; v.const_slope = 0.2f;
     v.out_buf = hr2; v.out_pitch = nf;
     P->add_conv(v);
+    // (NV12: the epilogue converts the uint8 RGB result itself on the streaming kernel; the engine falls back to a uint8
+    //  frame of its own + the rgb_to_nv12 kernel where this conv runs elsewhere)
     ConvSpec l = base_conv("conv_last", hr2, th * 4, tw * 4, nf, nf, 3);
     l.out_mode = om; l.out_buf = kBufExternalOut;
     P->add_conv(l);
@@ -207,10 +211,24 @@ void js_ks(std::ostringstream& o, const char* k, const std::string& v, bool last
 
 std::string build_bsvd_clip(const PlanCfgLite& c, Program* P);  // bsvd_program.cpp
 
+std::string nv12_out_check(const PlanCfgLite& cfg) {
+  if (cfg.out_fmt != 3) return "";
+  if (cfg.arch == 0) return "NV12 output is for RRDBNet plans: SRVGG's output feeds the colour-match glue (float / half NCHW)";
+  if (cfg.arch == 2) return "NV12 output is for RRDBNet plans: BSVD's output feeds the sharpen glue (float / half NCHW)";
+  if (cfg.arch != 1) return "";
+  const long long oh = static_cast<long long>(cfg.h) * cfg.scale, ow = static_cast<long long>(cfg.w) * cfg.scale;
+  if (oh % 2 || ow % 4) return "NV12 output needs an even output height and an output width divisible by 4";
+  return "";
+}
+
 std::string build_program(const PlanCfgLite& cfg, Program* out) {
   out->in_fmt = cfg.in_fmt;
   out->out_fmt = cfg.out_fmt;
   if (cfg.n < 1 || cfg.h < 1 || cfg.w < 1) return "bad frame geometry";
+  {
+    const std::string e = nv12_out_check(cfg);
+    if (!e.empty()) return e;
+  }
   switch (cfg.arch) {
     case 0: return build_srvgg(cfg, out);
     case 1: return build_rrdb(cfg, out);
@@ -245,6 +263,8 @@ std::string Program::to_json() const {
       js_kv(o, "w", p.w); js_kv(o, "n", p.n); js_kv(o, "n0", p.n0); js_kv(o, "unshuffle", p.unshuffle);
       js_kv(o, "out_buf", p.out_buf); js_kv(o, "out_lo_buf", p.out_lo_buf);
       js_kv(o, "fill_ch", p.fill_ch); js_kv(o, "fill_val", p.fill_val, true);
+    } else if (s.kind == 2) {
+      js_ks(o, "kind", "rgb_to_nv12", true);
     } else {
       const ConvSpec& c = s.conv;
       js_ks(o, "kind", "conv"); js_ks(o, "name", c.name); js_ks(o, "wname", c.wname);

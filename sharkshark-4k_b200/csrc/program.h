@@ -71,7 +71,8 @@ struct ConvSpec {
 };
 
 struct Step {
-  int kind = 0;  // 0 prep, 1 conv
+  int kind = 0;  // 0 prep, 1 conv, 2 uint8 RGB -> NV12 of the plan's output (added by the engine: NV12 output whose
+                 //   last conv does not store NV12 itself, engine.cu::ss4k_plan_create)
   PrepSpec prep;
   ConvSpec conv;
 };
@@ -108,5 +109,7 @@ struct PlanCfgLite {
 
 // returns "" on success, else an error message
 std::string build_program(const PlanCfgLite& cfg, Program* out);
+// out_fmt SS4K_FMT_NV12: RRDBNet only, output height even and width divisible by 4 ("" when fine or not NV12)
+std::string nv12_out_check(const PlanCfgLite& cfg);
 
 }  // namespace ss4k

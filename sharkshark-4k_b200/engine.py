@@ -200,7 +200,18 @@ class PlanCache:
         return key in self._d
 
 
-_OUT_DTYPES = {L.FMT_F32_NCHW: torch.float32, L.FMT_F16_NCHW: torch.float16, L.FMT_U8_NHWC: torch.uint8}
+_OUT_DTYPES = {L.FMT_F32_NCHW: torch.float32, L.FMT_F16_NCHW: torch.float16, L.FMT_U8_NHWC: torch.uint8,
+               L.FMT_NV12: torch.uint8}
+
+
+def out_shape_of(out_fmt, n, c, h, w):
+    """Shape of a plan's output tensor for ss4k_plan_out_shape's (n, c, h, w): NHWC for uint8 RGB, packed NV12 frames
+    [n, h*3/2, w] (Y plane, then interleaved UV) for NV12, NCHW otherwise."""
+    if out_fmt == L.FMT_U8_NHWC:
+        return (n, h, w, c)
+    if out_fmt == L.FMT_NV12:
+        return (n, h * 3 // 2, w)
+    return (n, c, h, w)
 
 
 class Plan:
@@ -224,8 +235,7 @@ class Plan:
         self.in_bytes, self.out_bytes = ib.value, ob.value
 
     def out_shape(self):
-        n, c, h, w = self.out_nchw
-        return (n, h, w, c) if self.cfg.out_fmt == L.FMT_U8_NHWC else (n, c, h, w)
+        return out_shape_of(self.cfg.out_fmt, *self.out_nchw)
 
     def new_output(self):
         return torch.empty(self.out_shape(), device=self.engine.device, dtype=_OUT_DTYPES[self.cfg.out_fmt])
@@ -258,7 +268,8 @@ class Plan:
     def profile(self, x, out=None):
         """One un-graphed run with a CUDA event between every step: list of (ms, flops, kind) per step
         (kind 0 layout/colour kernel, 1 row-streaming conv kernel, 2 tile conv kernel, 3 fused residual dense block =
-        five convs in one launch, 4 a conv that is part of the fused launch in front of it: no time of its own)."""
+        five convs in one launch, 4 a conv that is part of the fused launch in front of it: no time of its own).  An
+        NV12-output plan whose last conv does not store NV12 itself ends with the uint8 RGB -> NV12 conversion (kind 0)."""
         if out is None:
             out = self.new_output()
         cap = self.steps + 8

@@ -8,11 +8,16 @@ and the chunks sharded across GPUs with the 16-frame temporal halo (``sharding.b
     NV12 / uint8 RGB frames [T, ...]  --BSVD clip (T frames)-->  half NCHW [T,3,H,W]
         --owned frames: 0.8 * clamp(sharpen(denoised), 0, 1) + 0.2 * decoded frame   (fsrcnn_upscaler.py:278-281)
         -->  RRDBNet / SRVGG, one frame per engine run  -->  uint8 NHWC [n_own, sH, sW, 3]
+                                                             or NV12 [n_own, sH*3/2, sW] (RRDBNet, out_fmt=FMT_NV12)
 
 Both nets are engine plans (CUDA graphs of tcgen05 convs) behind the C ABI; colour decode, /255 and the noise map
 (0.1 * denoise_rate, fsrcnn_upscaler.py:262) are produced by the BSVD plan's layout kernel, the sharpen / clamp / blend
 between the nets by the service glue kernel (csrc/glue.cu, which decodes the NV12 frame for the blend itself).  torch
 supplies device buffers, streams and pinned host memory only.
+
+With ``out_fmt=FMT_NV12`` (RRDBNet upscalers) the frames leave as packed NV12 -- the Y plane then interleaved UV, the
+layout ``Engine.nv12_unpack`` hands to an encoder's surfaces -- converted by the upscaler's last convolution itself:
+bit-identical to the uint8 RGB result followed by ``Engine.rgb_to_nv12``, at half the bytes per frame.
 """
 import ctypes
 
@@ -55,14 +60,16 @@ class DenoiseUpscalePipeline:
         return tuple(self.sr_plan.out_shape()[1:])
 
     def new_output(self, n_own):
-        dt = {L.FMT_U8_NHWC: torch.uint8, L.FMT_F16_NCHW: torch.float16, L.FMT_F32_NCHW: torch.float32}[self.out_fmt]
+        dt = {L.FMT_U8_NHWC: torch.uint8, L.FMT_NV12: torch.uint8, L.FMT_F16_NCHW: torch.float16,
+              L.FMT_F32_NCHW: torch.float32}[self.out_fmt]
         return torch.empty((n_own,) + self.out_frame_shape(), device=self.device, dtype=dt)
 
 
     # ------------------------------------------------------------------ device-resident path
     def run(self, frames, own=None, out=None, after_frame=None):
         """frames: CUDA uint8 chunk [T, h*w*3/2] (NV12) or [T,h,w,3]; own: slice of the chunk whose frames are
-        upscaled (default: all); returns [n_own, sH, sW, 3] uint8 (stream-ordered, no sync)."""
+        upscaled (default: all); returns the upscaled frames in the pipeline's out_fmt: [n_own, sH, sW, 3] uint8 RGB,
+        [n_own, sH*3/2, sW] uint8 NV12, or [n_own, 3, sH, sW] float / half (stream-ordered, no sync)."""
         with torch.cuda.device(self.device):     # the glue kernel launches on the current device's stream
             return self._run(frames, own, out, after_frame)
 
@@ -105,7 +112,7 @@ class DenoiseUpscalePipeline:
 
     # ------------------------------------------------------------------ host path (pinned buffers in / out)
     def run_host(self, frames_host, own, out_host):
-        """Pinned host chunk in, pinned host frames out.  The H2D copy, both nets and the D2H copies are queued and the
+        """Pinned host chunk in, pinned host frames out (``out_host`` shaped like ``new_output``, any out_fmt).  The H2D copy, both nets and the D2H copies are queued and the
         call returns; the D2H copy of frame i overlaps the upscaling of frame i+1 (copy stream) and consecutive
         calls alternate between two device staging slots.  Call ``host_sync()`` before reading ``out_host``."""
         assert not frames_host.is_cuda and not out_host.is_cuda

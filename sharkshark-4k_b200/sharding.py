@@ -45,7 +45,9 @@ def bsvd_chunks(n_frames, world, halo=BSVD_HALO):
 
 def gather_frames(local, n_frames, dst=0, group=None):
     """Gather every rank's finished frames [n_local, ...] to ``dst`` in stream order.  Returns the full clip on
-    ``dst`` and None elsewhere.  Ranks may own different frame counts: shards are padded to the largest."""
+    ``dst`` and None elsewhere.  Ranks may own different frame counts: shards are padded to the largest.  Shape- and
+    dtype-generic past the frame dimension: uint8 RGB [n, H, W, 3], packed NV12 [n, H*3/2, W] (half the bytes) or float
+    frames gather the same way."""
     world = dist.get_world_size(group)
     rank = dist.get_rank(group)
     shards = frame_shards(n_frames, world)
