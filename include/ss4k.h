@@ -237,6 +237,19 @@ int ss4k_glue_finalize(const void* hr, int fmt, int n, int c, int h, int w, cons
 int ss4k_glue_finalize_bicubic_u8(const void* hr, int fmt, int n, int c, int h, int w, const float* diff, int dh, int dw,
                                   const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr,
                                   uint8_t* out_u8, int oh, int ow, int round_u8, void* cuda_stream);
+/* the two entries above with NV12 output for an encoder: packed frames [n, oh*3/2, ow] (Y plane u8[oh,ow], then
+ * interleaved UV u8[oh/2,ow]; the layout of in_fmt SS4K_FMT_NV12 and ss4k_nv12_unpack).  The bytes are exactly those of
+ * the uint8 entry with the same arguments (same truncation or round_u8 rounding) followed by ss4k_rgb_to_nv12 (BT.709
+ * limited range, 15-bit fixed point, chroma = mean of the 2x2 block), without the uint8 RGB frame.  SS4K_E_INVALID
+ * unless c == 3, the output height is even, the output width is a multiple of 4 and out_nv12 is 4-byte aligned; the
+ * geometry checks of the uint8 entries (diff sizes, the patch guard of the resizing form) apply unchanged.
+ * finalize_nv12: no resize, the output is (h, w); h, w, n >= 1. */
+int ss4k_glue_finalize_nv12(const void* hr, int fmt, int n, int c, int h, int w, const float* diff, int dh, int dw,
+                            const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr,
+                            uint8_t* out_nv12, int round_u8, void* cuda_stream);
+int ss4k_glue_finalize_bicubic_nv12(const void* hr, int fmt, int n, int c, int h, int w, const float* diff, int dh, int dw,
+                                    const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr,
+                                    uint8_t* out_nv12, int oh, int ow, int round_u8, void* cuda_stream);
 /* SS4K_E_INVALID unless n, c, h, w, oh, ow >= 1 */
 int ss4k_glue_bicubic_u8(const float* in, int n, int c, int h, int w, uint8_t* out, int oh, int ow, int round_u8,
                          void* cuda_stream);

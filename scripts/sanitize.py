@@ -30,6 +30,13 @@ print("service", tuple(sv.upscale(torch.randint(0, 256, (1, 72, 136, 3), dtype=t
 sv.output_shape = None
 print("service", tuple(sv.upscale(torch.randint(0, 256, (1, 72, 136, 3), dtype=torch.uint8).cuda()).shape))
 print("rgb->nv12", tuple(ss4k_b200.Engine.get(0).rgb_to_nv12(torch.randint(0, 256, (1, 8, 32, 3), dtype=torch.uint8).cuda()).shape))
+# NV12 output of the service glue: the fused finalise + bicubic store (ragged 32 x 8 tiles: 150 rows, 280 columns) and the
+# no-resize finalise store (ragged width), into buffers of exactly the frames' size
+sv.out_fmt = L.FMT_NV12
+sv.output_shape = (150, 280)
+print("service nv12", tuple(sv.upscale(torch.randint(0, 256, (2, 72, 136, 3), dtype=torch.uint8).cuda()).shape))
+sv.output_shape = None
+print("service nv12", tuple(sv.upscale(torch.randint(0, 256, (1, 18, 35, 3), dtype=torch.uint8).cuda()).shape))
 # round 2: frame decode in the first BSVD conv (decoder warps, NV12 and uint8 RGB, ragged width, owned range), split
 # precision twin-tile stores and specialised store paths, ring-buffer streaming (split, phase graphs), the cfg3 pipeline
 # with the glue writing the upscaler's first activation tensor, in-engine tiling, NV12 surfaces

@@ -77,6 +77,10 @@ SYMBOLS = {
                                 _i, _vp]),
     "ss4k_glue_finalize_bicubic_u8": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
                                            _i, _i, _i, _vp]),
+    "ss4k_glue_finalize_nv12": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp,
+                                     _i, _vp]),
+    "ss4k_glue_finalize_bicubic_nv12": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp, ctypes.c_double, ctypes.c_double,
+                                             _vp, _i, _i, _i, _vp]),
     "ss4k_glue_bicubic_u8": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _vp]),
     "ss4k_glue_sharpen_blend": (_i, [_vp, _i, _i, _i, _i, _i, ctypes.c_float, ctypes.c_float, _vp, _i, _vp, _vp]),
     "ss4k_glue_sharpen_blend_act": (_i, [_vp, _i, _i, _i, _i, _i, ctypes.c_float, ctypes.c_float, _vp, _i, _vp, _i, _i, _i, _vp]),

@@ -306,23 +306,24 @@ __global__ void bicubic_u8_kernel(const float* __restrict__ in, int N, int C, in
 //      bicubic from there.  Same arithmetic as finalize_kernel followed by bicubic_u8_kernel
 //      (fsrcnn_upscaler.py:214-233).  Source patch limit kFbMaxH x kFbMaxW (downscale factors up to 2).
 constexpr int kFbTw = 32, kFbTh = 8, kFbMaxW = 72, kFbMaxH = 24, kFbDiffRows = 6;
-__global__ void __launch_bounds__(kFbTw * kFbTh)
-finalize_bicubic_u8_kernel(Img hr, const float* __restrict__ diff, int dh, int dw, const double* hr_sums,
-                           const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* __restrict__ out,
-                           int OH, int OW, int round_u8) {
-  __shared__ float patch[3][kFbMaxH][kFbMaxW];
-  const int n = blockIdx.z;
-  const int ox0 = blockIdx.x * kFbTw, oy0 = blockIdx.y * kFbTh;
+// The tile's source patch, finalised into shared memory (both fused kernels): rows py0 .. and columns px0 .. of the
+// border-replicated image.  Every thread of the block calls this; it ends with a block-wide barrier.
+__device__ __forceinline__ void fb_stage_patch(const Img& hr, const float* __restrict__ diff, int dh, int dw, const double* hr_sums,
+                                               const double* lr_sums, double cnt_hr, double cnt_lr, int n, int OH, int OW,
+                                               int ox0, int oy0, float fy, float fx, int& py0_out, int& px0_out,
+                                               float (&patch)[3][kFbMaxH][kFbMaxW], float (&coef)[3][2],
+                                               float (&dxs)[3][kFbDiffRows][kFbMaxW], int (&col_x)[kFbMaxW]) {
   const int H = hr.H, W = hr.W;
-  const float fy = static_cast<float>(H) / OH, fx = static_cast<float>(W) / OW;
   // source patch: rows / columns touched by the taps of the tile's first and last output pixel (before clamping)
   const int oy1 = min(oy0 + kFbTh, OH) - 1, ox1 = min(ox0 + kFbTw, OW) - 1;
   const int py0 = static_cast<int>(floorf((oy0 + 0.5f) * fy - 0.5f)) - 1;
   const int py1 = static_cast<int>(floorf((oy1 + 0.5f) * fy - 0.5f)) + 2;
   const int px0 = static_cast<int>(floorf((ox0 + 0.5f) * fx - 0.5f)) - 1;
   const int px1 = static_cast<int>(floorf((ox1 + 0.5f) * fx - 0.5f)) + 2;
+  py0_out = py0;
+  px0_out = px0;
   const int ph = py1 - py0 + 1, pw = px1 - px0 + 1;  // host guarantees ph <= kFbMaxH, pw <= kFbMaxW
-  __shared__ float coef[3][2];  // match coefficients: double precision with square roots, once per block
+  // match coefficients (coef): double precision with square roots, once per block
   if (threadIdx.x < 3) match_coeffs(hr_sums, lr_sums, n * hr.C + threadIdx.x, cnt_hr, cnt_lr, &coef[threadIdx.x][0], &coef[threadIdx.x][1]);
   __syncthreads();
   const float ma[3] = {coef[0][0], coef[1][0], coef[2][0]}, mb[3] = {coef[0][1], coef[1][1], coef[2][1]};
@@ -330,8 +331,6 @@ finalize_bicubic_u8_kernel(Img hr, const float* __restrict__ diff, int dh, int d
   // patch touches along x once per column (dxs), then every patch element needs two shared-memory reads and one
   // lerp per channel instead of twelve global loads and nine lerps.  Same operations in the same order as
   // finalize_kernel (top / bottom row lerps along x, then the lerp along y), so the results are bit-identical.
-  __shared__ float dxs[3][kFbDiffRows][kFbMaxW];
-  __shared__ int col_x[kFbMaxW];
   int dy_lo = 0;
   bool staged = diff != nullptr;
   if (diff != nullptr) {
@@ -415,6 +414,21 @@ finalize_bicubic_u8_kernel(Img hr, const float* __restrict__ diff, int dh, int d
     for (int c = 0; c < 3; ++c) patch[c][ry][rx] = fminf(fmaxf(ma[c] * hr.at(n, c, y, x) + mb[c] - sub[c], 0.f), 1.f);
   }
   __syncthreads();
+}
+
+__global__ void __launch_bounds__(kFbTw * kFbTh)
+finalize_bicubic_u8_kernel(Img hr, const float* __restrict__ diff, int dh, int dw, const double* hr_sums,
+                           const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* __restrict__ out,
+                           int OH, int OW, int round_u8) {
+  __shared__ float patch[3][kFbMaxH][kFbMaxW];
+  __shared__ float coef[3][2];
+  __shared__ float dxs[3][kFbDiffRows][kFbMaxW];
+  __shared__ int col_x[kFbMaxW];
+  const int n = blockIdx.z;
+  const int ox0 = blockIdx.x * kFbTw, oy0 = blockIdx.y * kFbTh;
+  const float fy = static_cast<float>(hr.H) / OH, fx = static_cast<float>(hr.W) / OW;
+  int py0, px0;
+  fb_stage_patch(hr, diff, dh, dw, hr_sums, lr_sums, cnt_hr, cnt_lr, n, OH, OW, ox0, oy0, fy, fx, py0, px0, patch, coef, dxs, col_x);
   const int x = ox0 + (threadIdx.x % kFbTw), y = oy0 + (threadIdx.x / kFbTw);
   // a warp is one 32-pixel output row of the tile: packed word stores when the whole row is inside the image
   const bool live = x < OW && y < OH;
@@ -445,6 +459,128 @@ finalize_bicubic_u8_kernel(Img hr, const float* __restrict__ diff, int dh, int d
     else out[oidx * 3 + c] = static_cast<uint8_t>(f);
   }
   if (packed) store_rgb_row32(out + (oidx - (threadIdx.x & 31)) * 3, px);
+}
+
+// ---- NV12 output of the finalising kernels: the uint8 RGB bytes of the kernels above, converted with
+//      rgb_to_nv12_kernel's integer arithmetic (elementwise.cu: BT.709 limited range, 15-bit fixed point, chroma = mean
+//      of the 2x2 block) and stored as packed frames [N, OH*3/2, OW]: Y plane, then interleaved UV.
+// A block of kFbTw x kFbTh threads is a 32 x 8 tile of output pixels whose warp w is row oy0 + w (oy0 % 8 == 0), so the
+// two rows of a chroma pair are warps 2k and 2k+1.  Each warp stores its own Y row as packed words; the even warp leaves
+// its horizontal pair sums in `xchg`, and after one block-wide barrier the odd warp adds its own and stores the UV row.
+// Every thread of the block calls this, dead ones included (rgb then ignored).  OH % 2 == 0 and OW % 4 == 0: a row pair
+// is entirely inside or outside the image, and so is each group of 4 lanes.  frame: 4-byte aligned.
+__device__ __forceinline__ void store_nv12_tile(uint8_t* frame, int OH, int OW, int x, int y, bool live, const int rgb[3],
+                                                uint32_t (&xchg)[kFbTh / 2][kFbTw / 2]) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const uint32_t yv = static_cast<uint32_t>(16 + ((5983 * rgb[0] + 20127 * rgb[1] + 2032 * rgb[2] + 16384) >> 15));
+  uint32_t yw = yv | (__shfl_down_sync(0xffffffffu, yv, 1) << 8);
+  yw |= __shfl_down_sync(0xffffffffu, yw, 2) << 16;   // lane 4i: Y of pixels 4i .. 4i+3
+  const bool st_word = live && (lane & 3) == 0;
+  if (st_word) *reinterpret_cast<uint32_t*>(frame + static_cast<size_t>(y) * OW + x) = yw;
+  // R, G, B of the pixel pair (lanes 2i, 2i+1) as 10-bit fields: a 2x2 sum is at most 1020
+  const uint32_t hs1 = static_cast<uint32_t>(rgb[0]) | (static_cast<uint32_t>(rgb[1]) << 10) | (static_cast<uint32_t>(rgb[2]) << 20);
+  const uint32_t hs = hs1 + __shfl_xor_sync(0xffffffffu, hs1, 1);
+  uint32_t& slot = xchg[warp >> 1][lane >> 1];
+  if ((warp & 1) == 0 && (lane & 1) == 0) slot = hs;
+  __syncthreads();
+  if (warp & 1) {
+    const uint32_t s4 = hs + ((lane & 1) == 0 ? slot : 0u);   // lane 2i: the 2x2 block's sums
+    const int sr = static_cast<int>(s4 & 0x3FFu), sg = static_cast<int>((s4 >> 10) & 0x3FFu), sb = static_cast<int>(s4 >> 20);
+    const int uu = 128 + ((-3298 * sr - 11094 * sg + 14392 * sb + 65536) >> 17);
+    const int vv = 128 + ((14392 * sr - 13073 * sg - 1319 * sb + 65536) >> 17);
+    uint32_t uvw = (static_cast<uint32_t>(uu) & 0xFFu) | ((static_cast<uint32_t>(vv) & 0xFFu) << 8);
+    uvw |= __shfl_down_sync(0xffffffffu, uvw, 2) << 16;   // lane 4i: U, V of pairs 2i, 2i+1
+    if (st_word) *reinterpret_cast<uint32_t*>(frame + static_cast<size_t>(OH) * OW + static_cast<size_t>(y >> 1) * OW + x) = uvw;
+  }
+}
+
+// finalize_bicubic_u8_kernel with the NV12 store: same tile, patch staging and bicubic taps (same expressions in the
+// same order, so the same bytes before the conversion).  No early return: every thread reaches store_nv12_tile's barrier.
+__global__ void __launch_bounds__(kFbTw * kFbTh)
+finalize_bicubic_nv12_kernel(Img hr, const float* __restrict__ diff, int dh, int dw, const double* hr_sums,
+                             const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* __restrict__ out,
+                             int OH, int OW, int round_u8) {
+  __shared__ float patch[3][kFbMaxH][kFbMaxW];
+  __shared__ float coef[3][2];
+  __shared__ float dxs[3][kFbDiffRows][kFbMaxW];
+  __shared__ int col_x[kFbMaxW];
+  __shared__ uint32_t xchg[kFbTh / 2][kFbTw / 2];
+  const int n = blockIdx.z;
+  const int ox0 = blockIdx.x * kFbTw, oy0 = blockIdx.y * kFbTh;
+  const float fy = static_cast<float>(hr.H) / OH, fx = static_cast<float>(hr.W) / OW;
+  int py0, px0;
+  fb_stage_patch(hr, diff, dh, dw, hr_sums, lr_sums, cnt_hr, cnt_lr, n, OH, OW, ox0, oy0, fy, fx, py0, px0, patch, coef, dxs, col_x);
+  const int x = ox0 + (threadIdx.x % kFbTw), y = oy0 + (threadIdx.x / kFbTw);
+  const bool live = x < OW && y < OH;
+  int rgb[3] = {0, 0, 0};
+  if (live) {
+    const float A = -0.75f;
+    const float sy = (y + 0.5f) * fy - 0.5f, sx = (x + 0.5f) * fx - 0.5f;
+    const int iy = static_cast<int>(floorf(sy)), ix = static_cast<int>(floorf(sx));
+    const float ty = sy - iy, tx = sx - ix;
+    const float wy[4] = {cubic2(ty + 1.f, A), cubic1(ty, A), cubic1(1.f - ty, A), cubic2(2.f - ty, A)};
+    const float wx[4] = {cubic2(tx + 1.f, A), cubic1(tx, A), cubic1(1.f - tx, A), cubic2(2.f - tx, A)};
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      float acc = 0.f;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int ry = iy - 1 + j - py0;
+        float row = 0.f;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) row += wx[i] * patch[c][ry][ix - 1 + i - px0];
+        acc += wy[j] * row;
+      }
+      float f = fminf(fmaxf(acc, 0.f), 1.f) * 255.f;
+      if (round_u8) f = rintf(f);
+      rgb[c] = static_cast<uint8_t>(f);
+    }
+  }
+  store_nv12_tile(out + static_cast<size_t>(n) * OH * OW * 3 / 2, OH, OW, x, y, live, rgb, xchg);
+}
+
+// finalize_kernel's uint8 arithmetic (match affine, bilinear up-sampling of diff, clamp, x255, truncation or rint; same
+// expressions in the same order) on a 2-D grid of 32 x 8 tiles, blockIdx.z = image, with the NV12 store.  C == 3.
+__global__ void __launch_bounds__(kFbTw * kFbTh)
+finalize_nv12_kernel(Img hr, const float* __restrict__ diff, int dh, int dw, const double* hr_sums, const double* lr_sums,
+                     double cnt_hr, double cnt_lr, uint8_t* __restrict__ out, int round_u8) {
+  __shared__ float coef[3][2];
+  __shared__ uint32_t xchg[kFbTh / 2][kFbTw / 2];
+  const int n = blockIdx.z;
+  if (threadIdx.x < 3) match_coeffs(hr_sums, lr_sums, n * 3 + threadIdx.x, cnt_hr, cnt_lr, &coef[threadIdx.x][0], &coef[threadIdx.x][1]);
+  __syncthreads();
+  const int x = blockIdx.x * kFbTw + (threadIdx.x % kFbTw), y = blockIdx.y * kFbTh + (threadIdx.x / kFbTw);
+  const bool live = x < hr.W && y < hr.H;
+  int rgb[3] = {0, 0, 0};
+  if (live) {
+    int y0 = 0, y1 = 0, x0 = 0, x1 = 0;
+    float ly = 0.f, lx = 0.f;
+    if (diff != nullptr) {
+      float sy = (y + 0.5f) * (static_cast<float>(dh) / hr.H) - 0.5f;
+      float sx = (x + 0.5f) * (static_cast<float>(dw) / hr.W) - 0.5f;
+      sy = sy < 0.f ? 0.f : sy;
+      sx = sx < 0.f ? 0.f : sx;
+      y0 = static_cast<int>(sy); x0 = static_cast<int>(sx);
+      y1 = y0 < dh - 1 ? y0 + 1 : y0;
+      x1 = x0 < dw - 1 ? x0 + 1 : x0;
+      ly = sy - y0; lx = sx - x0;
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      float v = coef[c][0] * hr.at(n, c, y, x) + coef[c][1];
+      if (diff != nullptr) {
+        const float* d = diff + static_cast<size_t>(n * 3 + c) * dh * dw;
+        const float top = d[y0 * dw + x0] * (1.f - lx) + d[y0 * dw + x1] * lx;
+        const float bot = d[y1 * dw + x0] * (1.f - lx) + d[y1 * dw + x1] * lx;
+        v -= top * (1.f - ly) + bot * ly;
+      }
+      v = fminf(fmaxf(v, 0.f), 1.f);
+      float f = v * 255.f;
+      if (round_u8) f = rintf(f);
+      rgb[c] = static_cast<uint8_t>(f);
+    }
+  }
+  store_nv12_tile(out + static_cast<size_t>(n) * hr.H * hr.W * 3 / 2, hr.H, hr.W, x, y, live, rgb, xchg);
 }
 
 // ---- 3x3 depthwise reflect "sharpen" + clamp, optional blend with another image (float NCHW in/out) ----------
@@ -651,6 +787,32 @@ int ss4k_glue_finalize_bicubic_u8(const void* hr, int fmt, int n, int c, int h, 
   dim3 grid((ow + kFbTw - 1) / kFbTw, (oh + kFbTh - 1) / kFbTh, n);
   finalize_bicubic_u8_kernel<<<grid, kFbTw * kFbTh, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       Img{hr, fmt, n, c, h, w}, diff, dh, dw, hr_sums, lr_sums, cnt_hr, cnt_lr, out_u8, oh, ow, round_u8);
+  return cudaGetLastError() == cudaSuccess ? SS4K_OK : SS4K_E_CUDA;
+}
+
+int ss4k_glue_finalize_nv12(const void* hr, int fmt, int n, int c, int h, int w, const float* diff, int dh, int dw,
+                            const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* out_nv12,
+                            int round_u8, void* stream) {
+  if (!hr || !out_nv12 || fmt < 0 || fmt > 1 || c != 3 || n < 1 || h < 1 || w < 1) return SS4K_E_INVALID;
+  if (h % 2 || w % 4 || reinterpret_cast<uintptr_t>(out_nv12) % 4) return SS4K_E_INVALID;
+  if (diff && (dh < 1 || dw < 1)) return SS4K_E_INVALID;
+  dim3 grid((w + kFbTw - 1) / kFbTw, (h + kFbTh - 1) / kFbTh, n);
+  finalize_nv12_kernel<<<grid, kFbTw * kFbTh, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      Img{hr, fmt, n, c, h, w}, diff, dh, dw, hr_sums, lr_sums, cnt_hr, cnt_lr, out_nv12, round_u8);
+  return cudaGetLastError() == cudaSuccess ? SS4K_OK : SS4K_E_CUDA;
+}
+
+int ss4k_glue_finalize_bicubic_nv12(const void* hr, int fmt, int n, int c, int h, int w, const float* diff, int dh, int dw,
+                                    const double* hr_sums, const double* lr_sums, double cnt_hr, double cnt_lr, uint8_t* out_nv12,
+                                    int oh, int ow, int round_u8, void* stream) {
+  if (!hr || !out_nv12 || fmt < 0 || fmt > 1 || c != 3 || oh <= 0 || ow <= 0) return SS4K_E_INVALID;
+  if (oh % 2 || ow % 4 || reinterpret_cast<uintptr_t>(out_nv12) % 4) return SS4K_E_INVALID;
+  if (diff && (dh < 1 || dw < 1)) return SS4K_E_INVALID;
+  const double fy = static_cast<double>(h) / oh, fx = static_cast<double>(w) / ow;   // same patch guard as the uint8 entry
+  if (fy * (kFbTh - 1) + 5.0 > kFbMaxH || fx * (kFbTw - 1) + 5.0 > kFbMaxW) return SS4K_E_INVALID;
+  dim3 grid((ow + kFbTw - 1) / kFbTw, (oh + kFbTh - 1) / kFbTh, n);
+  finalize_bicubic_nv12_kernel<<<grid, kFbTw * kFbTh, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      Img{hr, fmt, n, c, h, w}, diff, dh, dw, hr_sums, lr_sums, cnt_hr, cnt_lr, out_nv12, oh, ow, round_u8);
   return cudaGetLastError() == cudaSuccess ? SS4K_OK : SS4K_E_CUDA;
 }
 

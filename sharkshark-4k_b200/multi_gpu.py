@@ -13,7 +13,10 @@ class keeps exactly that surface, so the unchanged orchestrator can drive a whol
     ``on_queue`` / ``get_result`` sees them -- the reference's single process produced them in order for free;
   * the reference's drop policy is kept: ``push_job_nowait`` raises ``queue.Full`` when the chosen worker's queue is
     full, and the dropped sequence number is skipped by the reorder buffer instead of stalling it;
-  * a worker that fails reports the exception; it is re-raised in the parent by the next call.
+  * a worker that fails reports the exception; it is re-raised in the parent by the next call;
+  * every other keyword goes to the workers' services unchanged: ``out_fmt=FMT_NV12`` makes them return packed NV12
+    frames ``uint8 [N, H*3/2, W]`` for an encoder.  The reorder buffer moves whole entries and never looks at the
+    frames' shape.
 
 The convnets need no collective (frames are independent, weights replicated); the temporal BSVD path shards as
 contiguous chunks with a 16-frame halo instead (``sharding.bsvd_chunks`` / ``sharding.StreamChunker``).

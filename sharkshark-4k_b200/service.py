@@ -3,7 +3,8 @@
 Reference: src/upscale/fsrcnn_upscaler.py:86-326 ``FsrcnnUpscalerService`` (+ src/upscale/upscaler_base.py:17-63).
 Same constructor keywords, same attributes (``lr_shape``, ``output_shape``, ``profiler``), same methods
 (``proc_init``, ``proc_cleanup``, ``upscale``, ``upscale_multi``, ``upscale_single``, ``proc_job_recieved``):
-``upscale(frames uint8 [N,H,W,3] on the device) -> uint8 [N,H',W',3]``.  The queue / process plumbing of
+``upscale(frames uint8 [N,H,W,3] on the device) -> uint8 [N,H',W',3]``, or with ``out_fmt=FMT_NV12`` packed NV12 frames
+``uint8 [N,H'*3/2,W']`` (Y plane, then interleaved UV) that an encoder surface takes as they are (``ss4k_nv12_unpack``).  The queue / process plumbing of
 ``BaseService`` is NOT re-implemented: in the reference tree this class is mixed into ``BaseUpscalerService``
 (see INTEGRATION.md); stand-alone it is driven by calling ``proc_init()`` then ``upscale()``.
 
@@ -56,6 +57,19 @@ def _fmt(t):
     return 1 if t.dtype == torch.float16 else 0
 
 
+def frame_shape(out_fmt, h, w):
+    """Shape of one output frame of (h, w) pixels: (h, w, 3) for uint8 RGB, (h*3/2, w) for packed NV12.  NV12 needs an
+    even height and a width divisible by 4; other sizes raise Ss4kError rather than yield a truncated frame."""
+    if out_fmt == L.FMT_U8_NHWC:
+        return (h, w, 3)
+    if out_fmt == L.FMT_NV12:
+        if h % 2 or w % 4:
+            raise L.Ss4kError(f"NV12 output needs an even height and a width divisible by 4, not {h}x{w} "
+                              "(set output_shape to such a size, or use out_fmt=FMT_U8_NHWC)")
+        return (h * 3 // 2, w)
+    raise ValueError(f"out_fmt must be FMT_U8_NHWC ({L.FMT_U8_NHWC}) or FMT_NV12 ({L.FMT_NV12}), not {out_fmt!r}")
+
+
 def gaussian_kernel(kernel_size=3, sigma=0.5):
     """blur_ker weights (fsrcnn_upscaler.py:20-52): normalised 2-D gaussian."""
     ax = torch.arange(kernel_size, dtype=torch.float32) - (kernel_size - 1) / 2.0
@@ -69,7 +83,9 @@ class FsrcnnUpscalerService:
     def __init__(self, lr_level=3, device=0, on_queue=None, denoising=True, denoise_rate=1.0,
                  upscaler_model='realesrgan', batch_size=1, jit_mode=None, lr_hr_resize=True,
                  model_name=None, state_dict=None, denoise_state_dict=None, act_mode=L.ACT_F16,
-                 denoise_act_mode="auto", single_mode=None, temporal_denoise=False):
+                 denoise_act_mode="auto", single_mode=None, temporal_denoise=False, out_fmt=L.FMT_U8_NHWC):
+        if out_fmt not in (L.FMT_U8_NHWC, L.FMT_NV12):
+            raise ValueError(f"out_fmt must be FMT_U8_NHWC ({L.FMT_U8_NHWC}) or FMT_NV12 ({L.FMT_NV12}), not {out_fmt!r}")
         self.lr_shape = self.LR_SHAPES[lr_level]
         self.scale = 4
         self.denoise_rate = denoise_rate
@@ -96,6 +112,9 @@ class FsrcnnUpscalerService:
         # 510-513) instead of one F = 1 clip per frame (fsrcnn_upscaler.py:277): every frame is denoised with its +-16
         # temporal neighbours and leaves the service 16 frames late (jobs are delayed as a whole, see proc_job_recieved)
         self.temporal_denoise = bool(temporal_denoise)
+        # out_fmt: frames leave as uint8 RGB [N,H,W,3] (the reference's) or as packed NV12 [N,H*3/2,W] for an encoder; the
+        # colour-match finalising kernel writes NV12 itself, so no separate conversion pass runs
+        self.out_fmt = out_fmt
         self.model = None
 
     # ------------------------------------------------------------------ life cycle (fsrcnn_upscaler.py:118-142)
@@ -163,9 +182,13 @@ class FsrcnnUpscalerService:
             frames = torch.stack([self._ready.popleft() for _ in range(n)], dim=0)
             return UpscalerQueueEntry(frames=frames, step=old.step, audio_segment=old.audio_segment, elapsed=elapsed,
                                       last_modified=time.time(), profiler=old.profiler)
-        oh, ow = self.output_shape if self.output_shape is not None else (0, 0)
-        return UpscalerQueueEntry(frames=torch.empty(0, oh, ow, 3, dtype=torch.uint8, device=self.device), step=-1,
+        return UpscalerQueueEntry(frames=self._no_frames(), step=-1,
                                   audio_segment=None, elapsed=elapsed, last_modified=time.time(), profiler=None)
+
+    def _no_frames(self):
+        """The frame-less result while the temporal pipeline fills: [0, *frame] of output_shape ((0, 0) while unset)."""
+        oh, ow = self.output_shape if self.output_shape is not None else (0, 0)
+        return torch.empty((0,) + frame_shape(self.out_fmt, oh, ow), dtype=torch.uint8, device=self.device)
 
     def flush(self):
         """End of the stream (temporal mode): drains BSVD's pipeline (the reference feeds None, bsvd/model.py:555-569) and
@@ -203,24 +226,34 @@ class FsrcnnUpscalerService:
         return out
 
     def _finish(self, hr, n, h, w, diff, hs, ls, cnt_hr, cnt_lr, want_resize):
+        """The colour-matched frames [n, *frame_shape] in out_fmt.  NV12: the finalising kernels store NV12 themselves
+        (fused resize: finalize_bicubic_nv12, no resize: finalize_nv12); the two-pass resize for downscale factors above
+        2 (e.g. lr_level 5: 4320p -> 1440p; off the live path) converts its uint8 RGB frame with Engine.rgb_to_nv12."""
         dh, dw = (diff.shape[-2], diff.shape[-1]) if diff is not None else (0, 0)
         st = self._stream()
+        nv12 = self.out_fmt == L.FMT_NV12
+        oh, ow = self.output_shape if want_resize else (h, w)
+        shape = (n,) + frame_shape(self.out_fmt, oh, ow)   # raises before any launch when NV12 cannot hold (oh, ow)
         if want_resize:
-            oh, ow = self.output_shape
-            out = torch.empty(n, oh, ow, 3, dtype=torch.uint8, device=self.device)
             if h <= 2 * oh and w <= 2 * ow:
+                out = torch.empty(shape, dtype=torch.uint8, device=self.device)
                 # clamp(match - colour diff) and the bicubic resize (:214-231) in one pass over the net's output
-                L.check(self.lib.ss4k_glue_finalize_bicubic_u8(_ptr(hr), _fmt(hr), n, 3, h, w, _ptr(diff), dh, dw, _ptr(hs),
-                                                               _ptr(ls), cnt_hr, cnt_lr, _ptr(out), oh, ow, 0, st))
+                entry = self.lib.ss4k_glue_finalize_bicubic_nv12 if nv12 else self.lib.ss4k_glue_finalize_bicubic_u8
+                L.check(entry(_ptr(hr), _fmt(hr), n, 3, h, w, _ptr(diff), dh, dw, _ptr(hs), _ptr(ls), cnt_hr, cnt_lr, _ptr(out),
+                              oh, ow, 0, st))
                 return out
             tmp = torch.empty(n, 3, h, w, dtype=torch.float32, device=self.device)   # downscale > 2: two passes
             L.check(self.lib.ss4k_glue_finalize(_ptr(hr), _fmt(hr), n, 3, h, w, _ptr(diff), dh, dw, _ptr(hs), _ptr(ls),
                                                 cnt_hr, cnt_lr, None, _ptr(tmp), 0, st))
-            L.check(self.lib.ss4k_glue_bicubic_u8(_ptr(tmp), n, 3, h, w, _ptr(out), oh, ow, 0, st))
-            return out
-        out = torch.empty(n, h, w, 3, dtype=torch.uint8, device=self.device)
-        L.check(self.lib.ss4k_glue_finalize(_ptr(hr), _fmt(hr), n, 3, h, w, _ptr(diff), dh, dw, _ptr(hs), _ptr(ls),
-                                            cnt_hr, cnt_lr, _ptr(out), None, 0, st))
+            rgb = torch.empty(n, oh, ow, 3, dtype=torch.uint8, device=self.device)
+            L.check(self.lib.ss4k_glue_bicubic_u8(_ptr(tmp), n, 3, h, w, _ptr(rgb), oh, ow, 0, st))
+            return self.engine.rgb_to_nv12(rgb).view(shape) if nv12 else rgb
+        out = torch.empty(shape, dtype=torch.uint8, device=self.device)
+        entry_args = (_ptr(hr), _fmt(hr), n, 3, h, w, _ptr(diff), dh, dw, _ptr(hs), _ptr(ls), cnt_hr, cnt_lr, _ptr(out))
+        if nv12:
+            L.check(self.lib.ss4k_glue_finalize_nv12(*entry_args, 0, st))
+        else:
+            L.check(self.lib.ss4k_glue_finalize(*entry_args, None, 0, st))
         return out
 
     def _run_model(self, lr):
@@ -273,8 +306,7 @@ class FsrcnnUpscalerService:
                 done.append(self._finish_single(den, self._lr_fifo.popleft()))
         if done:
             return torch.stack(done, dim=0)
-        oh, ow = self.output_shape if self.output_shape is not None else (0, 0)
-        return torch.empty(0, oh, ow, 3, dtype=torch.uint8, device=self.device)
+        return self._no_frames()
 
     def upscale_multi(self, img):
         """fsrcnn_upscaler.py:168-233"""
