@@ -135,13 +135,9 @@ double ss4k_plan_flops(const ss4k_plan* plan);
 int ss4k_plan_launches(const ss4k_plan* plan);
 /* how many of those steps replay from the plan's CUDA graph (0: graph capture unavailable / disabled) */
 int ss4k_plan_graph_steps(const ss4k_plan* plan);
-/* steps of the layer program (== entries ss4k_plan_profile returns; a fused residual dense block -- basicsr
- * ResidualDenseBlock, reached from realesrgan/factory.py:113-125 -- is five steps but one launch) */
+/* steps of the layer program (== entries ss4k_plan_profile returns; every step is one launch, except a layout step whose
+ * work the first conv's loader does, which launches nothing) */
 int ss4k_plan_steps(const ss4k_plan* plan);
-/* residual dense blocks that run as one fused launch each (0: the trunk runs conv by conv) */
-int ss4k_plan_fused_blocks(const ss4k_plan* plan);
-/* debug: per-CTA producer statistics of the fused launches of a plan created with SS4K_RDB_TRACE=1 */
-int64_t ss4k_debug_rdb_trace(ss4k_plan* plan, long long* out, int64_t cap);
 /* JSON description of the layer program (buffers, convs, epilogues); malloc'd, free with ss4k_free.
  * Works without a GPU when the plan was built with ss4k_plan_dry (host-side planner only). */
 int ss4k_plan_dry(const ss4k_plan_cfg* cfg, char** out_json);
@@ -164,8 +160,8 @@ int ss4k_plan_host_sync(ss4k_plan* plan);
 int ss4k_plan_io_bytes(const ss4k_plan* plan, int64_t* in_bytes, int64_t* out_bytes);
 /* measurement entry (bench.py roofline): one run of the plan without its CUDA graph, a CUDA event between
  * every step on `cuda_stream`.  ms[i] = device time of step i, flops[i] = its algorithmic FLOPs,
- * kind[i] = 0 layout/colour kernel, 1 row-streaming conv kernel, 2 tile conv kernel, 3 fused residual dense block,
- * 4 a conv inside the fused launch in front of it.  An NV12-output plan whose last conv does not store NV12 itself has
+ * kind[i] = 0 layout/colour kernel, 1 row-streaming conv kernel, 2 tile conv kernel, 4 a layout step done by the
+ * first conv's loader (no launch of its own).  An NV12-output plan whose last conv does not store NV12 itself has
  * one more step at the end: the uint8 RGB -> NV12 conversion (kind 0).  Returns the step count (<= cap) or a negative
  * error. */
 int ss4k_plan_profile(ss4k_plan* plan, const void* in_dev, void* out_dev, void* cuda_stream, float* ms,

@@ -50,8 +50,6 @@ SYMBOLS = {
     "ss4k_plan_graph_steps": (_i, [_vp]),
     "ss4k_plan_steps": (_i, [_vp]),
     "ss4k_debug_tile_layout": (_i, [_vp, ctypes.POINTER(ctypes.c_void_p)]),
-    "ss4k_plan_fused_blocks": (_i, [_vp]),
-    "ss4k_debug_rdb_trace": (_i64, [_vp, ctypes.POINTER(ctypes.c_longlong), _i64]),
     "ss4k_plan_dry": (_i, [ctypes.POINTER(PlanCfg), ctypes.POINTER(_vp)]),
     "ss4k_free": (None, [_vp]),
     "ss4k_run": (_i, [_vp, _vp, _vp, _vp]),

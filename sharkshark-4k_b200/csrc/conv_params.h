@@ -146,7 +146,6 @@ constexpr int kMaskRects = 16;                 // crops per atlas image
 constexpr int kMaskStride = 1 + 3 * kMaskRects;  // int32 words per image in StreamParams::mask_hw
 constexpr int kStreamSrcWarps = 2;  // frame-format source (StreamParams::src_fmt): decoder warps on top, alternating input rows
 constexpr int kStreamThreadsMax = kStreamThreads + 32 * kStreamSrcWarps;
-constexpr int kRdbThreads = kStreamThreads;                 // fused residual dense block kernel: same warp roles
 
 struct StreamParams {
   CUtensorMap tmA[2];   // 5-D (64, W, channel block, H, N), box (64, 130, 1, 1, 1), swizzle 128B
@@ -224,63 +223,6 @@ struct StreamParams {
   int32_t stride2;
   int32_t nkx;                // weight tiles (horizontal shifts) per K block: 3, or 2 for stride 2
   uint8_t ksm[kMaxSKB][2];    // stride 2: 4-bit mask of the 16-channel k-steps to issue per (K block, shift)
-};
-
-
-// ------------------------------------------------------------------------------------------------
-// Fused residual dense block (rdb_fused.cu): the five convs of one basicsr ResidualDenseBlock
-// (conv1..4: 64+32k -> 32 + LeakyReLU(0.2) into the slab's growth channels; conv5: 192 -> 64, x5*0.2 + x [+ RRDB residual])
-// as ONE persistent launch of six phases (conv5 = two 32-wide output chunks).  The frame is cut into column strips x
-// row bands with the SAME band boundaries in every strip, one CTA per (image, strip, band); a CTA keeps its band
-// through the phases and what one phase reads from an earlier one is guarded by per-CTA progress counters in global
-// memory instead of a kernel boundary.  Every other phase shifts the bands by half a band (the rows that fall off the
-// top wrap to the bottom of the same strip), so the rows a phase starts and ends with were produced in the MIDDLE of
-// the previous phase's bands: every dependency has about half a band of slack and the counters are never waited for.
-constexpr int kRdbPhases = 6;
-constexpr int kRdbNout = 32;
-constexpr int kRdbMaxWTiles = 9;     // K blocks x horizontal taps of the widest phase (192 input channels)
-constexpr int kRdbCtrPerCta = 8;     // one progress counter per epilogue warp
-
-struct RdbPhase {
-  int32_t nkb;          // 64-channel K blocks read by this conv
-  int32_t nks_last;     // 16-channel k-steps of the last K block (the others issue 4)
-  int32_t w_row0;       // first row of the phase's weight tiles in the packed weight tensor
-  int32_t bias0;        // offset of the phase's bias in bias_f
-  int32_t out_c0;       // first output channel in the destination tensor (TMA store coordinate)
-  int32_t out_map;      // 0: this block's slab, 1: the next block's slab
-  int32_t dep;          // the phase whose output rows this one reads (its newest input channels), -1: none
-  int32_t shift;        // 1: bands shifted up by `half` rows (wrapping inside the strip)
-  int32_t residual;     // 0: LeakyReLU epilogue; 1: linear + residual adds (conv5), residual channel offset res_c
-  int32_t res_c;
-  int32_t l2_in, l2_out;
-};
-
-struct RdbParams {
-  CUtensorMap tmA;      // this block's slab, 5-D (64, W, channel block, H, N), box (64, 130, 1, 1, 1), swizzle 128B
-  CUtensorMap tmW;      // packed weights of the five convs, 2-D (64, rows), box (64, 96)
-  CUtensorMap tmO[2];   // 4-D (C, W, H, N), box (32, 32, 1, 1), swizzle 64B: this slab / the next slab
-  RdbPhase ph[kRdbPhases];
-  const float* bias_f;  // fp32 bias of every phase, alpha folded in (the accumulators' initial value)
-  float slope;          // LeakyReLU slope of conv1..4
-  float beta1, beta2;   // conv5: out = acc + beta1 * res1 + beta2 * res2
-  const void* res1;     // this slab's x (NHWC 16-bit, pitch res1_pitch)
-  const void* res2;     // the RRDB input (third block of an RRDB), or null
-  int32_t res1_pitch, res1_coff, res2_pitch, res2_coff;
-  int32_t n_img, H, W, strips;
-  int32_t bands;        // row bands per strip: grid = n_img * strips * bands, CTA = (n * strips + strip) * bands + band
-  int32_t half;         // rows by which the shifted phases move the bands
-  int32_t acc_slots, a_slots;
-  uint32_t idesc[3];
-  uint32_t* ctr_use;    // progress counters of this launch: [grid][kRdbCtrPerCta] rows completed per epilogue warp
-  uint32_t* ctr_zero;   // the buffer the NEXT fused launch uses: cleared by this one
-  void* discard_ptr;    // dead-tensor discard (see StreamParams)
-  uint32_t discard_pitch_bytes, discard_mask;
-  int64_t discard_npx;
-  const void* next_w;   // packed weights of the next launch (L2 prefetch), or null
-  uint32_t next_w_bytes;
-  int32_t* err;
-  int32_t dbg_flags;    // 1: ignore the progress counters (WRONG results; measures what the dependency waits cost)
-  long long* trace;     // debug: per-CTA producer statistics [grid][16] (polls, clocks waiting for counters / slabs, phase start clocks); null in production
 };
 
 }  // namespace ss4k

@@ -15,11 +15,6 @@ cudaError_t conv_stream_prepare();
 cudaError_t conv_stream_launch(const StreamParams& p, int nout, int grid, cudaStream_t stream, bool pdl);
 int conv_stream_max_ctas_per_sm(int nout);  // resident CTAs per SM of the variant (early activation loads need exactly 1)
 
-// rdb_fused.cu: the five convs of a residual dense block as one persistent launch
-cudaError_t rdb_fused_prepare();
-int rdb_fused_max_ctas_per_sm();
-cudaError_t rdb_fused_launch(const RdbParams& p, int grid, cudaStream_t stream, bool pdl);
-
 // tiled inference: one padded crop of the (reflect-padded) frame and where its un-padded centre goes in the output
 struct TileBox {
   int32_t src_y, src_x;       // top-left of the padded crop in the input frame

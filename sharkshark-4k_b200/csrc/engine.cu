@@ -120,10 +120,6 @@ struct DeviceGuard {
 struct ConvExec {
   ConvParams p;
   StreamParams sp;      // row-streaming kernel (conv_stream.cu) when `stream` is set
-  RdbParams rp;         // fused residual dense block (rdb_fused.cu) when `fused` is set: this step launches conv1..5
-  bool fused = false;
-  bool skip = false;    // conv2..5 of a fused block: no launch of their own
-  double fused_flops = 0;
   bool stream = false;
   int nout = 0;         // accumulator slot width of the streaming kernel
   int grid = 0;
@@ -786,8 +782,6 @@ int materialize_stream(ss4k_ctx* ctx, const ConvSpec& cs, const HostTensor& W, c
 const bool g_use_pdl = getenv("SS4K_NO_PDL") == nullptr;
 
 cudaError_t launch_exec(const ConvExec& c, void* ext_out, cudaStream_t st) {
-  if (c.skip) return cudaSuccess;
-  if (c.fused) return rdb_fused_launch(c.rp, c.grid, st, g_use_pdl);
   if (c.stream) {
     if (c.ext_out) {
       StreamParams p = c.sp;
@@ -892,9 +886,6 @@ struct ss4k_plan {
   int graph_first = -1, graph_last = -1;  // [first, last] step range inside the graph
   int fused_prep = -1;   // step index of a layout (prep) step whose work the following conv's loader does, or -1
   int32_t* d_mask = nullptr;  // masked canvases (cfg.reserved[5]): crop size (h, w) of every image of the batch at the input resolution
-  uint32_t* d_ctr = nullptr;  // progress counters of the fused residual dense blocks (3 rotating buffers)
-  long long* d_rdb_trace = nullptr;  // SS4K_RDB_TRACE=1: producer statistics of every fused launch [n_fused][nsm][16]
-  int n_fused = 0;
   void* stage_in = nullptr;   // device staging for ss4k_run_host
   void* stage_out = nullptr;
   // NV12 output in two steps (tiled plans, or a last conv that does not run on the streaming kernel): the uint8 RGB frame
@@ -957,167 +948,11 @@ int run_step(ss4k_plan* pl, int si, const void* in_dev, void* out_dev, cudaStrea
     ctx->launches++;
   } else {
     ConvExec& c = pl->convs[pl->step_conv[si]];
-    if (c.skip) return SS4K_OK;
     if (c.src_ext) c.sp.src = reinterpret_cast<const uint8_t*>(in_dev) + c.src_off;
     // (two-step NV12 output: the last conv writes the plan's uint8 RGB frame, the conversion step the caller's buffer)
     CK(ctx, launch_exec(c, c.ext_out && pl->nv12_rgb != nullptr ? pl->nv12_rgb : out_dev, st));
     ctx->launches++;
   }
-  return SS4K_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-// Fused residual dense blocks: every run of five trunk convs body.B.rdbR.conv1..conv5 becomes one launch of
-// rdb_fused_kernel (rdb_fused.cu).  Built from the five materialised streaming convs: their packed weights and biases
-// are concatenated, their tensor maps / epilogue constants re-used.
-int fuse_rdbs(ss4k_plan* pl) {
-  ss4k_ctx* ctx = pl->ctx;
-  // Opt-in (SS4K_RDB_FUSE=1): measured on B200 the fused launch is correct (bit-identical) but not faster than the
-  // conv-by-conv trunk with programmatic dependent launch -- the convs are bound by the shared-memory port inside every
-  // row, not by their boundaries (DESIGN.md section 4.6, profiles/r02_*).
-  const char* fuse_env = getenv("SS4K_RDB_FUSE");
-  if (fuse_env == nullptr || atoi(fuse_env) == 0 || pl->cfg.act_mode != SS4K_ACT_F16) return SS4K_OK;
-  if (rdb_fused_max_ctas_per_sm() != 1) return SS4K_OK;   // the progress-counter waits need one co-resident CTA per SM
-  Program& P = pl->prog;
-  const int ns = static_cast<int>(P.steps.size());
-  std::vector<int> groups;
-  auto ends_with = [](const std::string& a, const std::string& b) { return a.size() >= b.size() && a.compare(a.size() - b.size(), b.size(), b) == 0; };
-  for (int si = 0; si + 4 < ns; ++si) {
-    if (P.steps[si].kind != 1) continue;
-    const std::string& nm = P.steps[si].conv.name;
-    if (nm.rfind("body.", 0) != 0 || !ends_with(nm, ".conv1")) continue;
-    const std::string pre = nm.substr(0, nm.size() - 1);
-    bool ok = true;
-    for (int k = 0; k < 5 && ok; ++k) {
-      const Step& st = P.steps[si + k];
-      if (st.kind != 1 || st.conv.name != pre + std::to_string(k + 1)) { ok = false; break; }
-      const ConvExec& c = pl->convs[pl->step_conv[si + k]];
-      const ConvSpec& cs = st.conv;
-      ok = c.stream && !c.fused && !c.skip && c.nout == kRdbNout && !cs.split && c.grid == ctx->nsm && c.sp.fast_store == 1 &&
-           c.sp.chunks == (k == 4 ? 2 : 1) && cs.in_buf == P.steps[si].conv.in_buf && cs.in_coff == 0 &&
-           cs.cin == 64 + 32 * k && cs.in_pitch == 192 && cs.out_pitch == 192 && !c.sp.stride2 &&
-           (k == 4 ? (cs.out_coff == 0 && cs.res1_buf == cs.in_buf) : (cs.out_buf == cs.in_buf && cs.out_coff == 64 + 32 * k));
-    }
-    if (!ok) continue;
-    const StreamParams& s0 = pl->convs[pl->step_conv[si]].sp;
-    // strips x bands with the same band boundaries in every strip, one CTA per (image, strip, band): worth it only if
-    // that grid fills the GPU and a band has a few rows on each side of the half-band shift
-    const int nstrip = s0.n_img * s0.strips;
-    const int bands = nstrip > 0 ? std::min(ctx->nsm / nstrip, s0.H / 4) : 0;
-    if (bands < 1 || nstrip * bands * 100 < ctx->nsm * 94) continue;
-    groups.push_back(si);
-    si += 4;
-  }
-  const int ng = static_cast<int>(groups.size());
-  if (ng < 2) return SS4K_OK;
-  const size_t ctr_elems = static_cast<size_t>(ctx->nsm) * kRdbCtrPerCta;
-  CK(ctx, cudaMalloc(&pl->d_ctr, 3 * ctr_elems * sizeof(uint32_t)));
-  CK(ctx, cudaMemset(pl->d_ctr, 0, 3 * ctr_elems * sizeof(uint32_t)));
-  if (getenv("SS4K_RDB_TRACE") != nullptr) {
-    CK(ctx, cudaMalloc(&pl->d_rdb_trace, static_cast<size_t>(ng) * ctx->nsm * 16 * sizeof(long long)));
-    CK(ctx, cudaMemset(pl->d_rdb_trace, 0, static_cast<size_t>(ng) * ctx->nsm * 16 * sizeof(long long)));
-  }
-  // counter buffer of launch g: g % 3, except that the last launch must also differ from the first (graph replay wraps)
-  auto buf_of = [&](int g) { return (g == ng - 1 && ng % 3 == 1) ? 1 : g % 3; };
-  const CUtensorMapDataType dt = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  for (int gi = 0; gi < ng; ++gi) {
-    const int si = groups[gi];
-    ConvExec* c[5];
-    for (int k = 0; k < 5; ++k) c[k] = &pl->convs[pl->step_conv[si + k]];
-    const ConvSpec& cs1 = P.steps[si].conv;
-    const ConvSpec& cs5 = P.steps[si + 4].conv;
-    RdbParams rp;
-    memset(&rp, 0, sizeof(rp));
-    // ---- weights and biases of the five convs, back to back
-    size_t wtot = 0, btot = 0;
-    for (int k = 0; k < 5; ++k) { wtot += c[k]->w_bytes; btot += static_cast<size_t>(c[k]->sp.chunks) * kRdbNout; }
-    void* d_w = nullptr;
-    float* d_b = nullptr;
-    CK(ctx, cudaMalloc(&d_w, wtot));
-    CK(ctx, cudaMalloc(&d_b, btot * sizeof(float)));
-    size_t woff = 0, boff = 0;
-    double flops = 0;
-    int np = 0;   // phases: conv1..4, then conv5's two 32-wide output chunks
-    for (int k = 0; k < 5; ++k) {
-      CK(ctx, cudaMemcpy(reinterpret_cast<uint8_t*>(d_w) + woff, c[k]->d_w, c[k]->w_bytes, cudaMemcpyDeviceToDevice));
-      const size_t nb = static_cast<size_t>(c[k]->sp.chunks) * kRdbNout;
-      CK(ctx, cudaMemcpy(d_b + boff, c[k]->d_bias, nb * sizeof(float), cudaMemcpyDeviceToDevice));
-      const StreamParams& sp = c[k]->sp;
-      for (int kb = 0; kb + 1 < sp.nkb; ++kb)
-        if (sp.nks[kb] != 4) return fail(ctx, SS4K_E_INVALID, "fuse_rdbs: partial K block in front of the last one");
-      if (sp.nkb * 3 > kRdbMaxWTiles) return fail(ctx, SS4K_E_INVALID, "fuse_rdbs: too many weight tiles");
-      const size_t chunk_rows = static_cast<size_t>(sp.nkb) * 9 * kRdbNout;   // [kb][kx][2-ky][32] rows of 64 channels
-      for (int ch = 0; ch < sp.chunks; ++ch, ++np) {
-        RdbPhase& ph = rp.ph[np];
-        ph.nkb = sp.nkb;
-        ph.nks_last = sp.nks[sp.nkb - 1];
-        ph.w_row0 = static_cast<int32_t>(woff / 128 + ch * chunk_rows);
-        ph.bias0 = static_cast<int32_t>(boff) + ch * kRdbNout;
-        ph.out_c0 = P.steps[si + k].conv.out_coff + ch * kRdbNout;
-        ph.out_map = k == 4 ? 1 : 0;
-        ph.dep = k == 0 ? -1 : k - 1;     // conv(k+1) reads what conv(k) wrote; both chunks of conv5 read conv4's rows
-        ph.shift = (np & 1) && k < 4 ? 1 : 0;
-        ph.residual = k == 4 ? 1 : 0;
-        ph.res_c = ch * kRdbNout;
-        ph.l2_in = sp.l2_in; ph.l2_out = sp.l2_out;
-      }
-      woff += c[k]->w_bytes;
-      boff += nb;
-      flops += P.steps[si + k].conv.flops();
-    }
-    if (np != kRdbPhases) return fail(ctx, SS4K_E_INVALID, "fuse_rdbs: unexpected phase count");
-    rp.tmA = c[4]->sp.tmA[0];   // conv5 reads all three 64-channel blocks of the slab
-    {
-      cuuint64_t dims[2] = {64, static_cast<cuuint64_t>(wtot / 128)};
-      cuuint64_t strides[1] = {128};
-      cuuint32_t box[2] = {64, static_cast<cuuint32_t>(3 * kRdbNout)};
-      cuuint32_t es[2] = {1, 1};
-      CUresult r = ctx->encode(&rp.tmW, dt, 2, d_w, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(ctx, SS4K_E_CUDA, fmt("cuTensorMapEncodeTiled(fused weights) failed: %d", (int)r));
-    }
-    for (int m = 0; m < 2; ++m) {  // whole-slab output maps: this block's slab (growth channels), the next block's slab (x)
-      const ConvSpec& cs = m == 0 ? cs1 : cs5;
-      const cuuint64_t eb = 2;
-      cuuint64_t dims[4] = {static_cast<cuuint64_t>(cs.out_pitch), static_cast<cuuint64_t>(cs.out_w), static_cast<cuuint64_t>(cs.out_h),
-                            static_cast<cuuint64_t>(cs.n)};
-      cuuint64_t strides[3] = {cs.out_pitch * eb, static_cast<cuuint64_t>(cs.out_w) * cs.out_pitch * eb,
-                               static_cast<cuuint64_t>(cs.out_h) * cs.out_w * cs.out_pitch * eb};
-      cuuint32_t box[4] = {static_cast<cuuint32_t>(kRdbNout), 32, 1, 1};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      CUresult r = ctx->encode(&rp.tmO[m], dt, 4, pl->bufs[cs.out_buf], dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                               CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(ctx, SS4K_E_CUDA, fmt("cuTensorMapEncodeTiled(fused output) failed: %d", (int)r));
-    }
-    rp.bias_f = d_b;
-    rp.slope = c[0]->sp.ep.slope_const;
-    const Epilogue& e5 = c[4]->sp.ep;
-    rp.beta1 = e5.beta1; rp.beta2 = e5.beta2;
-    rp.res1 = e5.res1; rp.res1_pitch = e5.res1_pitch; rp.res1_coff = e5.res1_coff;
-    rp.res2 = e5.res2; rp.res2_pitch = e5.res2_pitch; rp.res2_coff = e5.res2_coff;
-    rp.n_img = c[0]->sp.n_img; rp.H = c[0]->sp.H; rp.W = c[0]->sp.W; rp.strips = c[0]->sp.strips;
-    rp.bands = std::min(ctx->nsm / (rp.n_img * rp.strips), rp.H / 4);
-    rp.half = (rp.H / rp.bands) / 2;
-    rp.acc_slots = c[0]->sp.acc_slots;
-    rp.a_slots = std::min(kMaxSASlots, (kSmemBytes - 2048 - kRdbMaxWTiles * 3 * kRdbNout * 128 - kStreamBiasBytes -
-                                        kStreamEpiWarps * round_up(32 * kRdbNout * 2, 1024)) / kASlotBytes);
-    for (int i = 0; i < 3; ++i) rp.idesc[i] = c[0]->sp.idesc[i];
-    rp.ctr_use = pl->d_ctr + static_cast<size_t>(buf_of(gi)) * ctr_elems;
-    rp.ctr_zero = pl->d_ctr + static_cast<size_t>(buf_of((gi + 1) % ng)) * ctr_elems;
-    rp.discard_ptr = c[0]->sp.discard_ptr; rp.discard_pitch_bytes = c[0]->sp.discard_pitch_bytes;
-    rp.discard_mask = c[0]->sp.discard_mask; rp.discard_npx = c[0]->sp.discard_npx;
-    rp.err = ctx->err_dev;
-    if (const char* e = getenv("SS4K_RDB_DBG")) rp.dbg_flags = atoi(e);
-    if (pl->d_rdb_trace != nullptr) rp.trace = pl->d_rdb_trace + static_cast<size_t>(gi) * ctx->nsm * 16;
-    // the group's first exec now owns the fused weights; the others launch nothing
-    for (int k = 0; k < 5; ++k) { free_conv(*c[k]); c[k]->skip = k > 0; c[k]->sp.next_w = nullptr; }
-    c[0]->fused = true;
-    c[0]->fused_flops = flops;
-    c[0]->rp = rp;
-    c[0]->d_w = d_w; c[0]->w_bytes = wtot; c[0]->d_bias = d_b;
-    c[0]->grid = rp.n_img * rp.strips * rp.bands;
-  }
-  pl->n_fused = ng;
   return SS4K_OK;
 }
 
@@ -1143,7 +978,7 @@ void fuse_prep(ss4k_plan* pl) {
   if (pl->cfg.act_mode == SS4K_ACT_BF16) return;
   if (pp.fill_ch >= 0 && pp.fill_ch != 3) return;
   ConvExec& c = pl->convs[pl->step_conv[1]];
-  if (!c.stream || c.fused || c.skip) return;
+  if (!c.stream) return;
   // the conv must cover every frame the layout step would have converted for other readers (the residual of the block's
   // last conv): its frame range contains theirs by construction (bsvd_program.cpp), check it anyway
   const int c0 = cs.n0, c1 = cs.n0 + cs.n;
@@ -1207,7 +1042,6 @@ int ss4k_create(int device_id, ss4k_ctx** out_ctx) {
   CK(nullptr, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
   CK(nullptr, conv_tc_prepare());
   CK(nullptr, conv_stream_prepare());
-  CK(nullptr, rdb_fused_prepare());
   const char* force = getenv("SS4K_DESC_MODE");
   if (force && *force) {
     ctx->desc_mode = atoi(force);
@@ -1315,8 +1149,6 @@ int ss4k_plan_destroy(ss4k_plan* pl) {
   if (pl->stage_in) cudaFree(pl->stage_in);
   if (pl->stage_out) cudaFree(pl->stage_out);
   if (pl->nv12_rgb) cudaFree(pl->nv12_rgb);
-  if (pl->d_ctr) cudaFree(pl->d_ctr);
-  if (pl->d_rdb_trace) cudaFree(pl->d_rdb_trace);
   if (pl->d_mask) cudaFree(pl->d_mask);
   delete pl;
   return SS4K_OK;
@@ -1395,10 +1227,6 @@ int ss4k_plan_create(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_pl
     P.steps.push_back(s);
     pl->step_conv.push_back(-1);
   }
-  {
-    int rc = fuse_rdbs(pl.get());
-    if (rc != SS4K_OK) { ss4k_plan_destroy(pl.release()); return rc; }
-  }
   fuse_prep(pl.get());
   if (cfg->reserved[5] == 1) {
     // masked canvases (tiled inference): every conv zeroes its output outside the image's crop; needs every conv on the
@@ -1416,7 +1244,7 @@ int ss4k_plan_create(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_pl
       const ConvSpec& cs = P.steps[si].conv;
       ConvExec& c = pl->convs[pl->step_conv[si]];
       int shift = 0, hh = P.in_h;
-      bool ok = c.stream && !c.fused && !c.skip && cs.mode == kModeConv3 && cs.n == P.in_n;
+      bool ok = c.stream && cs.mode == kModeConv3 && cs.n == P.in_n;
       if (ok) {
         while (hh < cs.in_h && shift < 4) { hh *= 2; ++shift; }
         while (hh > cs.in_h && shift > -4) { if (hh & 1) { ok = false; break; } hh /= 2; --shift; }
@@ -1438,7 +1266,6 @@ int ss4k_plan_create(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_pl
       const ConvExec& p1 = pl->convs[pl->step_conv[si - 1]];
       const ConvExec& p2 = pl->convs[pl->step_conv[si - 2]];
       const ConvSpec& cs = P.steps[si].conv;
-      if (c.fused || c.skip || p1.fused || p1.skip || p2.fused || p2.skip) continue;
       if (!c.stream || !p1.stream || !p2.stream || c.grid != ctx->nsm || p1.grid != ctx->nsm || p2.grid != ctx->nsm) continue;
       if (cs.old_cin <= 0 || cs.split) continue;
       // the argument above needs exactly one resident CTA per SM
@@ -1451,16 +1278,12 @@ int ss4k_plan_create(ss4k_ctx* ctx, const ss4k_plan_cfg* cfg, ss4k_plan** out_pl
   }
   // each launch prefetches the next launch's packed weights into L2 (the last one: the first conv's, for the next frame)
   if (getenv("SS4K_NO_W_PREFETCH") == nullptr) {
-    std::vector<ConvExec*> live;
-    for (auto& c : pl->convs)
-      if (!c.skip) live.push_back(&c);
-    const int nc = static_cast<int>(live.size());
+    const int nc = static_cast<int>(pl->convs.size());
     for (int i = 0; i < nc; ++i) {
-      ConvExec& c = *live[i];
-      const ConvExec& nx = *live[(i + 1) % nc];
-      if (nc < 2 || nx.d_w == nullptr || !(nx.stream || nx.fused)) continue;
-      if (c.fused) { c.rp.next_w = nx.d_w; c.rp.next_w_bytes = static_cast<uint32_t>(nx.w_bytes); }
-      else if (c.stream) { c.sp.next_w = nx.d_w; c.sp.next_w_bytes = static_cast<uint32_t>(nx.w_bytes); }
+      ConvExec& c = pl->convs[i];
+      const ConvExec& nx = pl->convs[(i + 1) % nc];
+      if (nc < 2 || !c.stream || nx.d_w == nullptr || !nx.stream) continue;
+      c.sp.next_w = nx.d_w; c.sp.next_w_bytes = static_cast<uint32_t>(nx.w_bytes);
     }
   }
   pl->in_bytes = fmt_bytes(P.in_fmt, P.in_n, P.in_c, P.in_h, P.in_w);
@@ -1733,10 +1556,10 @@ double ss4k_plan_flops(const ss4k_plan* pl) { return pl ? pl->prog.flops : 0.0; 
 static int live_steps(const ss4k_plan* pl, int first, int last) {
   int n = 0;
   for (int si = first; si <= last; ++si)
-    if (!(pl->prog.steps[si].kind == 1 && pl->convs[pl->step_conv[si]].skip) && si != pl->fused_prep) ++n;
+    if (si != pl->fused_prep) ++n;
   return n;
 }
-// kernels one run launches (a fused residual dense block is one launch for five convs)
+// kernels one run launches (a layout step done by the first conv's loader launches nothing)
 int ss4k_plan_launches(const ss4k_plan* pl) {
   if (!pl) return 0;
   int n = live_steps(pl, 0, static_cast<int>(pl->prog.steps.size()) - 1);
@@ -1751,16 +1574,6 @@ int ss4k_plan_graph_steps(const ss4k_plan* pl) {
   return n;
 }
 int ss4k_plan_steps(const ss4k_plan* pl) { return pl ? static_cast<int>(pl->prog.steps.size()) : 0; }
-int ss4k_plan_fused_blocks(const ss4k_plan* pl) { return pl ? pl->n_fused : 0; }
-// debug (plans created with SS4K_RDB_TRACE=1): producer statistics of the fused launches, [n_fused][nsm][16] int64
-int64_t ss4k_debug_rdb_trace(ss4k_plan* pl, long long* out, int64_t cap) {
-  if (!pl || !out || pl->d_rdb_trace == nullptr) return 0;
-  const int64_t n = static_cast<int64_t>(pl->n_fused) * pl->ctx->nsm * 16;
-  if (cap < n) return -n;
-  if (cudaDeviceSynchronize() != cudaSuccess) return 0;
-  if (cudaMemcpy(out, pl->d_rdb_trace, n * sizeof(long long), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
-  return n;
-}
 int ss4k_plan_io_bytes(const ss4k_plan* pl, int64_t* in_bytes, int64_t* out_bytes) {
   if (!pl) return SS4K_E_INVALID;
   if (in_bytes) *in_bytes = pl->in_bytes;
@@ -1906,7 +1719,8 @@ int ss4k_plan_host_sync(ss4k_plan* pl) {
 }
 
 // Per-step timing of one plan run (no CUDA graph): a CUDA event between every step on `cuda_stream`.
-// kind[i]: 0 prep / layout kernel, 1 row-streaming conv kernel, 2 tile conv kernel.  Returns the number of steps.
+// kind[i]: 0 prep / layout kernel, 1 row-streaming conv kernel, 2 tile conv kernel, 4 a layout step done by the first
+// conv's loader.  Returns the number of steps.
 int ss4k_plan_profile(ss4k_plan* pl, const void* in_dev, void* out_dev, void* cuda_stream, float* ms, double* flops,
                       int32_t* kind, int cap) {
   if (!pl || !in_dev || !out_dev || !ms || !flops || !kind) return fail(pl ? pl->ctx : nullptr, SS4K_E_INVALID, "null argument to ss4k_plan_profile");
@@ -1931,11 +1745,6 @@ int ss4k_plan_profile(ss4k_plan* pl, const void* in_dev, void* out_dev, void* cu
     flops[si] = s.kind == 1 ? s.conv.flops() : 0.0;
     if (s.kind == 2) { kind[si] = 0; continue; }   // the NV12 conversion of a two-step NV12 output: a colour kernel
     kind[si] = s.kind == 0 ? (si == pl->fused_prep ? 4 : 0) : (pl->convs[pl->step_conv[si]].stream ? 1 : 2);
-    if (s.kind == 1) {
-      const ConvExec& c = pl->convs[pl->step_conv[si]];
-      if (c.fused) { kind[si] = 3; flops[si] = c.fused_flops; }   // one launch for the block's five convs
-      else if (c.skip) { kind[si] = 4; flops[si] = 0.0; }         // part of the fused launch in front of it
-    }
   }
   for (auto& e : ev) cudaEventDestroy(e);
   return rc == SS4K_OK ? ns : rc;

@@ -229,7 +229,6 @@ class Plan:
         self.launches = self.lib.ss4k_plan_launches(h)
         self.graph_steps = self.lib.ss4k_plan_graph_steps(h)
         self.steps = self.lib.ss4k_plan_steps(h)
-        self.fused_blocks = self.lib.ss4k_plan_fused_blocks(h)
         ib, ob = ctypes.c_int64(), ctypes.c_int64()
         self.lib.ss4k_plan_io_bytes(h, ctypes.byref(ib), ctypes.byref(ob))
         self.in_bytes, self.out_bytes = ib.value, ob.value
@@ -267,9 +266,8 @@ class Plan:
 
     def profile(self, x, out=None):
         """One un-graphed run with a CUDA event between every step: list of (ms, flops, kind) per step
-        (kind 0 layout/colour kernel, 1 row-streaming conv kernel, 2 tile conv kernel, 3 fused residual dense block =
-        five convs in one launch, 4 a conv that is part of the fused launch in front of it: no time of its own).  An
-        NV12-output plan whose last conv does not store NV12 itself ends with the uint8 RGB -> NV12 conversion (kind 0)."""
+        (kind 0 layout/colour kernel, 1 row-streaming conv kernel, 2 tile conv kernel, 4 a layout step done by the
+        first conv's loader: no launch of its own).  An NV12-output plan whose last conv does not store NV12 itself ends with the uint8 RGB -> NV12 conversion (kind 0)."""
         if out is None:
             out = self.new_output()
         cap = self.steps + 8
