@@ -194,13 +194,22 @@ int ss4k_nv12_unpack(ss4k_ctx* ctx, const void* packed_dev, const ss4k_nv12_surf
  * layers active, no clip boundary in reach) replays one captured CUDA graph per phase of the longest ring between a copy
  * into and a copy out of stream-owned staging buffers (plan cfg use_graph = 0 or SS4K_NO_STREAM_GRAPH: per-layer launches). */
 int ss4k_bsvd_stream_open(ss4k_plan* plan, ss4k_bsvd_stream** out_stream);
+/* like ss4k_bsvd_stream_open, for pushes of up to max_frames (>= 1) frames per call.  Every conv of the streaming kernel
+ * then runs once over the frames of a push, its ring slots wrapping inside the kernel.  Each ring holds max_frames - 1
+ * more frames (lengths still rounded up to powers of two); max_frames = 1 is ss4k_bsvd_stream_open.  Steady-state
+ * pushes replay one graph per (phase, frame count). */
+int ss4k_bsvd_stream_open_batched(ss4k_plan* plan, int max_frames, ss4k_bsvd_stream** out_stream);
 /* push frame t (in_dev: one frame in the plan's in_fmt: 4 channels RGB + noise map for the float / half NCHW formats, a
  * uint8 RGB or NV12 frame for the frame formats -- the noise map is then the plan's reserved[0] level).
  * *got_output = 1 when the denoised frame t-16 was written to out_dev (3 channels). */
 int ss4k_bsvd_stream_push(ss4k_bsvd_stream* s, const void* in_dev, void* out_dev,
                           int* got_output, void* cuda_stream);
+/* push frames t .. t+n-1 (1 <= n <= max_frames; in_dev: n frames back to back in the plan's in_fmt); out_dev has room for
+ * n frames of 3 channels; *n_out = number of denoised frames written, oldest first (frames t-16 .. t+n-17 that exist).
+ * n outside [1, max_frames], a null pointer or a push after flush without reset: SS4K_E_INVALID. */
+int ss4k_bsvd_stream_push_frames(ss4k_bsvd_stream* s, const void* in_dev, int n, void* out_dev, int* n_out, void* cuda_stream);
 /* flush: feed "None" (end-of-clip) steps until the next denoised frame falls out of the pipeline;
- * call until *got_output == 0 (all frames of the clip delivered) */
+ * call until *got_output == 0 (all frames of the clip delivered; one frame per call, whatever the pushes carried) */
 int ss4k_bsvd_stream_flush(ss4k_bsvd_stream* s, void* out_dev, int* got_output, void* cuda_stream);
 int ss4k_bsvd_stream_reset(ss4k_bsvd_stream* s);
 /* frames of latency between a push and its output (BSVD.count_shift, model.py:582-588: 16) */
@@ -269,6 +278,10 @@ int ss4k_run_act(ss4k_plan* plan, void* out_dev, void* cuda_stream);
 /* host-only: the tile grid of a plan configuration (tile, tile_pad, reserved[1] = pre_pad) and its packing into crop
  * atlases as JSON; free with ss4k_free */
 int ss4k_debug_tile_layout(const ss4k_plan_cfg* cfg, char** out_json);
+/* host-only: a BSVD stream's layout for pushes of up to max_frames frames as JSON -- shift_num, period, every buffer's
+ * ring length and producer lag, every step's lag, buffers read / written and whether it scatters (temporal shift); free
+ * with ss4k_free */
+int ss4k_debug_bsvd_stream_layout(const ss4k_plan_cfg* cfg, int max_frames, char** out_json);
 
 /* operator-level entry (kernel parity tests) -------------------------------------------- */
 typedef struct ss4k_conv_desc {

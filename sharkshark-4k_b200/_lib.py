@@ -50,6 +50,7 @@ SYMBOLS = {
     "ss4k_plan_graph_steps": (_i, [_vp]),
     "ss4k_plan_steps": (_i, [_vp]),
     "ss4k_debug_tile_layout": (_i, [_vp, ctypes.POINTER(ctypes.c_void_p)]),
+    "ss4k_debug_bsvd_stream_layout": (_i, [_vp, _i, ctypes.POINTER(ctypes.c_void_p)]),
     "ss4k_plan_dry": (_i, [ctypes.POINTER(PlanCfg), ctypes.POINTER(_vp)]),
     "ss4k_free": (None, [_vp]),
     "ss4k_run": (_i, [_vp, _vp, _vp, _vp]),
@@ -60,7 +61,9 @@ SYMBOLS = {
     "ss4k_plan_profile": (_i, [_vp, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_double),
                                ctypes.POINTER(ctypes.c_int32), _i]),
     "ss4k_bsvd_stream_open": (_i, [_vp, ctypes.POINTER(_vp)]),
+    "ss4k_bsvd_stream_open_batched": (_i, [_vp, _i, ctypes.POINTER(_vp)]),
     "ss4k_bsvd_stream_push": (_i, [_vp, _vp, _vp, ctypes.POINTER(_i), _vp]),
+    "ss4k_bsvd_stream_push_frames": (_i, [_vp, _vp, _i, _vp, ctypes.POINTER(_i), _vp]),
     "ss4k_bsvd_stream_flush": (_i, [_vp, _vp, ctypes.POINTER(_i), _vp]),
     "ss4k_bsvd_stream_reset": (_i, [_vp]),
     "ss4k_bsvd_stream_latency": (_i, [_vp]),

@@ -111,11 +111,12 @@ class NativeBSVD(nn.Module):
         out = self._plan(n * f, h, w, in_fmt, out_fmt).run(x)
         return out.reshape(n, f, 3, h, w)
 
-    def stream(self, h, w, in_fmt=L.FMT_F32_NCHW, noise=0.0):
+    def stream(self, h, w, in_fmt=L.FMT_F32_NCHW, noise=0.0, max_frames=1):
         """A frame-at-a-time stream in this model's precision mode (the split precision mode included).  ``in_fmt``:
         ``FMT_F32_NCHW`` frames ``[4,h,w]`` (RGB + noise map, the reference layout) or ``FMT_U8_NHWC`` / ``FMT_NV12``
-        frames with the constant noise map ``noise`` filled in by the layout kernel."""
-        return BSVDStream(self, h, w, in_fmt, noise)
+        frames with the constant noise map ``noise`` filled in by the layout kernel.  ``max_frames``: the most frames one
+        ``push_frames`` call may carry (every ring then holds ``max_frames - 1`` more frames)."""
+        return BSVDStream(self, h, w, in_fmt, noise, max_frames)
 
     def streaming_forward(self, input_seq):
         """BSVD.streaming_forward (model.py:526-580) through the ring-buffer engine: feed, drain, reset."""
@@ -156,15 +157,16 @@ class NativeBSVD(nn.Module):
 class BSVDStream:
     """Frame-at-a-time denoising with persistent ring buffers in HBM (BSVD.feedin_one_element, model.py:510-513):
     ``push(frame)`` returns the denoised frame t-16 once the 16-stage pipeline is full, else None; ``flush()``
-    yields the remaining frames (the reference feeds ``None``, model.py:555-569); ``reset()`` starts a new clip."""
+    yields the remaining frames (the reference feeds ``None``, model.py:555-569); ``reset()`` starts a new clip.
+    ``push_frames(frames)`` pushes up to ``max_frames`` consecutive frames in one call (each conv runs once over them)."""
 
-    def __init__(self, model, h, w, in_fmt=L.FMT_F32_NCHW, noise=0.0):
+    def __init__(self, model, h, w, in_fmt=L.FMT_F32_NCHW, noise=0.0, max_frames=1):
         import ctypes
-        self.model, self.h, self.w, self.in_fmt = model, h, w, in_fmt
+        self.model, self.h, self.w, self.in_fmt, self.max_frames = model, h, w, in_fmt, max_frames
         self.lib = model.engine.lib
         self.plan = model._plan(1, h, w, in_fmt, L.FMT_F32_NCHW, noise)
         hdl = ctypes.c_void_p()
-        L.check(self.lib.ss4k_bsvd_stream_open(self.plan.h, ctypes.byref(hdl)), model.engine.h)
+        L.check(self.lib.ss4k_bsvd_stream_open_batched(self.plan.h, max_frames, ctypes.byref(hdl)), model.engine.h)
         self.hdl = hdl
         self.latency = self.lib.ss4k_bsvd_stream_latency(hdl)
 
@@ -185,6 +187,23 @@ class BSVDStream:
         L.check(self.lib.ss4k_bsvd_stream_push(self.hdl, ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(out.data_ptr()),
                                                ctypes.byref(got), self._st(x.device)), self.model.engine.h)
         return out if got.value else None
+
+    def push_frames(self, frames):
+        """Frames t .. t+n-1 of the stream: ``[n,4,h,w]`` float, ``[n,h,w,3]`` uint8 RGB or ``[n,h*3/2,w]`` NV12, with
+        1 <= n <= max_frames.  Returns the denoised frames that fell out, oldest first: ``[m,3,h,w]`` float, m may be 0."""
+        import ctypes
+        n = frames.shape[0]
+        if self.in_fmt == L.FMT_F32_NCHW:
+            x = frames.reshape(n, 4, self.h, self.w).float().contiguous()
+        else:
+            if frames.dtype != torch.uint8:
+                raise ValueError("frame-format streams take uint8 frames")
+            x = frames.contiguous()
+        out = torch.empty(n, 3, self.h, self.w, device=x.device, dtype=torch.float32)
+        got = ctypes.c_int(0)
+        L.check(self.lib.ss4k_bsvd_stream_push_frames(self.hdl, ctypes.c_void_p(x.data_ptr()), n, ctypes.c_void_p(out.data_ptr()),
+                                                      ctypes.byref(got), self._st(x.device)), self.model.engine.h)
+        return out[:got.value]
 
     def flush(self):
         import ctypes

@@ -299,11 +299,21 @@ __device__ __forceinline__ void store8_lo(void* base, size_t elem_off, const flo
   store8(base, elem_off, r, bf16);
 }
 
+// Where one output image of a launch lives: its image index in the output and residual tensors (relative to their base
+// pointers), its frame index in the clip (temporal-shift boundary guards) and the distances, in frames, to the
+// neighbouring frames' images (E.off_prev / E.off_next are one frame each).  They all follow from the launch's image
+// index n, except where a tensor is a ring of frames that wraps inside the launch (BSVD streams, conv_stream.cu::ring_img).
+struct ImgAt {
+  int out, res1, res2, t, prev, next;
+};
+__device__ __forceinline__ ImgAt img_at(const Epilogue& E, int n) { return ImgAt{n, n, n, E.t0 + n, 1, 1}; }
+
 // One 16-channel chunk of one output pixel: bias, activation, residuals, store.
 //   ch0: channel index of v[0] within the conv's (padded) output channels
 //   (ay, ax): pixel in A space; sub: accumulator phase (kModeUp2)
-__device__ __forceinline__ void epilogue_chunk(const Epilogue& E, int mode, int n, int ay, int ax, int sub,
+__device__ __forceinline__ void epilogue_chunk(const Epilogue& E, int mode, const ImgAt& I, int ay, int ax, int sub,
                                                int ch0, float (&v)[16]) {
+  const int n = I.out;
   const bool bf16 = E.is_bf16 != 0;
   // ---- bias + activation
   {
@@ -357,25 +367,27 @@ __device__ __forceinline__ void epilogue_chunk(const Epilogue& E, int mode, int 
   const size_t pix = (static_cast<size_t>(n) * E.out_h + oy) * E.out_w + ox;
   // ---- residuals (indexed at the output pixel, NHWC)
   if (E.res1 != nullptr) {
+    const size_t p1 = (static_cast<size_t>(I.res1) * E.out_h + oy) * E.out_w + ox;
     if (E.res1_nch > 0) {
       if (oc < E.res1_nch) {
         float r[16];
 #pragma unroll
         for (int i = 0; i < 16; ++i) r[i] = 0.f;
-        add_residual16(r, E.res1, pix * E.res1_pitch + E.res1_coff + oc, E.beta1, bf16);
-        if (E.res1_lo_off != 0) add_residual16(r, E.res1, pix * E.res1_pitch + E.res1_coff + oc + E.res1_lo_off, E.beta1, bf16);
+        add_residual16(r, E.res1, p1 * E.res1_pitch + E.res1_coff + oc, E.beta1, bf16);
+        if (E.res1_lo_off != 0) add_residual16(r, E.res1, p1 * E.res1_pitch + E.res1_coff + oc + E.res1_lo_off, E.beta1, bf16);
 #pragma unroll
         for (int i = 0; i < 16; ++i)
           if (oc + i < E.res1_nch) v[i] += r[i];
       }
     } else {
-      add_residual16(v, E.res1, pix * E.res1_pitch + E.res1_coff + oc, E.beta1, bf16);
-      if (E.res1_lo_off != 0) add_residual16(v, E.res1, pix * E.res1_pitch + E.res1_coff + oc + E.res1_lo_off, E.beta1, bf16);
+      add_residual16(v, E.res1, p1 * E.res1_pitch + E.res1_coff + oc, E.beta1, bf16);
+      if (E.res1_lo_off != 0) add_residual16(v, E.res1, p1 * E.res1_pitch + E.res1_coff + oc + E.res1_lo_off, E.beta1, bf16);
     }
   }
   if (E.res2 != nullptr) {
-    add_residual16(v, E.res2, pix * E.res2_pitch + E.res2_coff + oc, E.beta2, bf16);
-    if (E.res2_lo_off != 0) add_residual16(v, E.res2, pix * E.res2_pitch + E.res2_coff + oc + E.res2_lo_off, E.beta2, bf16);
+    const size_t p2 = (static_cast<size_t>(I.res2) * E.out_h + oy) * E.out_w + ox;
+    add_residual16(v, E.res2, p2 * E.res2_pitch + E.res2_coff + oc, E.beta2, bf16);
+    if (E.res2_lo_off != 0) add_residual16(v, E.res2, p2 * E.res2_pitch + E.res2_coff + oc + E.res2_lo_off, E.beta2, bf16);
   }
   // ---- store
   switch (E.out_mode) {
@@ -386,11 +398,11 @@ __device__ __forceinline__ void epilogue_chunk(const Epilogue& E, int mode, int 
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
           const int c = oc + 8 * h;
-          const int t = E.t0 + n;
+          const int t = I.t;
           int64_t delta = 0;
           bool ok = true;
-          if (c < E.fold) { delta = E.off_prev; ok = t > 0; }
-          else if (c < 2 * E.fold) { delta = E.off_next; ok = t < E.t_count - 1; }
+          if (c < E.fold) { delta = E.off_prev * I.prev; ok = t > 0; }
+          else if (c < 2 * E.fold) { delta = E.off_next * I.next; ok = t < E.t_count - 1; }
           if (ok) {
             const size_t o2 = static_cast<size_t>(static_cast<int64_t>(off) + 8 * h + delta);
             store8(E.out, o2, v + 8 * h, bf16);

@@ -192,7 +192,12 @@ struct StreamParams {
   int32_t dbg_flags;      // profiling experiments (scripts/bench_conv.py, SS4K_DBG_FLAGS): 1 skip MMA issue, 2 skip TMA
                           // loads, 4 epilogue without math / stores, 8 skip band halo rows (WRONG results), 16 full
                           // completion wait on the last output tiles, 64 trace rows stamped by epilogue warp 2
-  int32_t n_in0, n_out0;  // added to the image coordinate of TMA loads / stores (BSVD streaming: ring slots)
+  int32_t n_in0, n_out0;  // added to the image coordinate of TMA loads / stores (BSVD streaming: the frame of image 0)
+  // BSVD streams: each tensor is a ring of R frames (R a power of two), and a launch over several frames wraps around it.
+  // Image n of the launch lives in slot (n_in0 + n) & ring_in of the input tensor, (n_out0 + n) & ring_out of the output
+  // tensor, (n_out0 + n) & ring_res1 / ring_res2 of the residual tensors (mask R - 1; -1 for every other plan: no wrap).
+  // The epilogue's pointers (out, out_lo, res1, res2) are at image 0's slot of their tensor.
+  int32_t ring_in, ring_out, ring_res1, ring_res2;
   long long* trace;       // debug: per-CTA clock64 stamps [grid][64] (null in production)
   const void* next_w;     // packed weights of the next kernel of the plan (L2 prefetch), or null
   uint32_t next_w_bytes;

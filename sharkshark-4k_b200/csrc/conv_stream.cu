@@ -127,6 +127,23 @@ __device__ __forceinline__ bool next_band(const StreamParams& P, int& u, int u1,
   return true;
 }
 
+// Image n of the launch in the ring buffers of a BSVD stream (StreamParams::ring_*): the output / residual image indices
+// relative to the epilogue's base pointers, and the distances to frames n-1 / n+1 in the output ring (they wrap with it).
+// Every other plan has masks of -1: image n, one frame either side.
+__device__ __forceinline__ int ring_n(const StreamParams& P, int n, int mask) { return ((P.n_out0 + n) & mask) - (P.n_out0 & mask); }
+__device__ __forceinline__ ImgAt ring_img(const StreamParams& P, int n) {
+  const int f = P.n_out0 + n;
+  const int so = f & P.ring_out;
+  ImgAt I;
+  I.out = so - (P.n_out0 & P.ring_out);
+  I.res1 = ring_n(P, n, P.ring_res1);
+  I.res2 = ring_n(P, n, P.ring_res2);
+  I.t = P.ep.t0 + n;
+  I.prev = so - ((f - 1) & P.ring_out);
+  I.next = ((f + 1) & P.ring_out) - so;
+  return I;
+}
+
 }  // namespace
 
 static_assert(kMaxSASlots <= 16 && kMaxAccSlots <= 16, "barrier set-up assigns one lane per ring slot");
@@ -496,7 +513,7 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
               mbar_arrive(a_full + 8 * as);
             } else {
               mbar_expect_tx(a_full + 8 * as, kBoxW * kRowBytes);
-              tma_load_5d_hint(a_base + as * kASlotBytes, &P.tmA[P.a_tm[kb]], a_full + 8 * as, 0, x0, P.a_kb[kb], r, b.n + P.n_in0, pol_in);
+              tma_load_5d_hint(a_base + as * kASlotBytes, &P.tmA[P.a_tm[kb]], a_full + 8 * as, 0, x0, P.a_kb[kb], r, (b.n + P.n_in0) & P.ring_in, pol_in);
             }
           }
           if (ptr8) trace[114] = clock64();
@@ -688,7 +705,7 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
     bool have_next = false;
     while (next_band(P, u, u1, b)) {
       const int r0 = b.yb > 0 ? b.yb - 1 : b.yb, r1 = b.ye < P.H ? b.ye : b.ye - 1;
-      const int n_abs = b.n + P.n_in0;
+      const int n_abs = b.n + P.n_in0;   // (clip plans only: BSVD streams convert their frames in a layout step)
       const int xs = b.strip * kTileW, x4 = xs + 4 * lane;
       have_next = false;
       constexpr int kAhead = 8;   // rows between the L2 prefetch and the load
@@ -830,7 +847,8 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
           uint4 r1v[NOUT / 8], r2v[NOUT / 8];
           constexpr bool kPs2 = NOUT <= 32;          // (the planner uses the PixelShuffle(2) fast store with chunks <= 32 only)
           uint4 r1l[kPs2 ? NOUT / 8 : 1];            // split precision + PixelShuffle(2): low halves of the skip tensor
-          const size_t pix = (static_cast<size_t>(b.n) * E.out_h + y) * E.out_w + ax;
+          const int nr1 = ring_n(P, b.n, P.ring_res1);
+          const size_t pix1 = (static_cast<size_t>(nr1) * E.out_h + y) * E.out_w + ax;
           const bool has_r1 = fast && E.res1 != nullptr, has_r2 = fast && E.res2 != nullptr;
           // PixelShuffle(2) fast store: this chunk is (part of) sub-pixel phase ab of the shuffled tensor (channels
           // pre-permuted to (a, b, c)); E.out_h / E.out_w are the shuffled sizes
@@ -842,7 +860,7 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
             ps_c0 = b.chunk * NOUT - ps_ab * cq;
           }
           if (ps2 && has_r1 && valid) {
-            const size_t po = (static_cast<size_t>(b.n) * E.out_h + 2 * y + (ps_ab >> 1)) * E.out_w + 2 * ax + (ps_ab & 1);
+            const size_t po = (static_cast<size_t>(nr1) * E.out_h + 2 * y + (ps_ab >> 1)) * E.out_w + 2 * ax + (ps_ab & 1);
             const uint16_t* const rb = reinterpret_cast<const uint16_t*>(E.res1) + po * E.res1_pitch + E.res1_coff + ps_c0;
 #pragma unroll
             for (int j = 0; j < NOUT / 8; ++j) r1v[j] = reinterpret_cast<const uint4*>(rb)[j];
@@ -857,7 +875,7 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
 #pragma unroll
               for (int j = 0; j < NOUT / 8; ++j) r1v[j] = make_uint4(0u, 0u, 0u, 0u);
               if (b.chunk == 0) {
-                uint4 t = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(E.res1) + pix * E.res1_pitch + E.res1_coff);
+                uint4 t = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(E.res1) + pix1 * E.res1_pitch + E.res1_coff);
                 const int nch = E.res1_nch;
                 t.x &= (nch > 0 ? 0xFFFFu : 0u) | (nch > 1 ? 0xFFFF0000u : 0u);
                 t.y &= (nch > 2 ? 0xFFFFu : 0u) | (nch > 3 ? 0xFFFF0000u : 0u);
@@ -866,13 +884,13 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                 r1v[0] = t;
               }
             } else {
-              const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(E.res1) + pix * E.res1_pitch + E.res1_coff + b.chunk * NOUT);
+              const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(E.res1) + pix1 * E.res1_pitch + E.res1_coff + b.chunk * NOUT);
 #pragma unroll
               for (int j = 0; j < NOUT / 8; ++j) r1v[j] = rp[j];
             }
           }
           if (has_r2 && valid) {
-            const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(E.res2) + pix * E.res2_pitch + E.res2_coff + b.chunk * NOUT);
+            const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(E.res2) + ((static_cast<size_t>(ring_n(P, b.n, P.ring_res2)) * E.out_h + y) * E.out_w + ax) * E.res2_pitch + E.res2_coff + b.chunk * NOUT);
 #pragma unroll
             for (int j = 0; j < NOUT / 8; ++j) r2v[j] = rp[j];
           }
@@ -1063,18 +1081,19 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                 if (P.fast_store == 2) {
 #pragma unroll
                   for (int ab = 0; ab < 4; ++ab)
-                    tma_store_5d(&P.tmO, stage, b.chunk * NOUT, ab & 1, b.strip * kTileW + qd * 32, ab >> 1, (b.n + P.n_out0) * P.H + y, pol_out);
+                    tma_store_5d(&P.tmO, stage, b.chunk * NOUT, ab & 1, b.strip * kTileW + qd * 32, ab >> 1, ((b.n + P.n_out0) & P.ring_out) * P.H + y, pol_out);
                 } else if (ps2) {
-                  tma_store_5d(&P.tmO, stage, ps_c0, ps_ab & 1, b.strip * kTileW + qd * 32, ps_ab >> 1, (b.n + P.n_out0) * P.H + y, pol_out);
-                  if (split_store) tma_store_5d(&P.tmO2, stage + kStageWarp, ps_c0, ps_ab & 1, b.strip * kTileW + qd * 32, ps_ab >> 1, (b.n + P.n_out0) * P.H + y, pol_out);
+                  tma_store_5d(&P.tmO, stage, ps_c0, ps_ab & 1, b.strip * kTileW + qd * 32, ps_ab >> 1, ((b.n + P.n_out0) & P.ring_out) * P.H + y, pol_out);
+                  if (split_store) tma_store_5d(&P.tmO2, stage + kStageWarp, ps_c0, ps_ab & 1, b.strip * kTileW + qd * 32, ps_ab >> 1, ((b.n + P.n_out0) & P.ring_out) * P.H + y, pol_out);
                 } else {
-                  tma_store_4d(&P.tmO, stage, b.chunk * NOUT, b.strip * kTileW + qd * 32, y, b.n + P.n_out0, pol_out);
-                  if (split_store) tma_store_4d(&P.tmO2, stage + kStageWarp, b.chunk * NOUT, b.strip * kTileW + qd * 32, y, b.n + P.n_out0, pol_out);
+                  tma_store_4d(&P.tmO, stage, b.chunk * NOUT, b.strip * kTileW + qd * 32, y, (b.n + P.n_out0) & P.ring_out, pol_out);
+                  if (split_store) tma_store_4d(&P.tmO2, stage + kStageWarp, b.chunk * NOUT, b.strip * kTileW + qd * 32, y, (b.n + P.n_out0) & P.ring_out, pol_out);
                 }
                 bulk_commit();
               }
             } else if (NOUT == 16 && E.out_mode == kOutNV12) {
               if constexpr (NOUT == 16) {
+                const ImgAt I = ring_img(P, b.n);
                 // NV12 frame store (RRDBNet's conv_last, out_fmt SS4K_FMT_NV12): the bytes of the kOutU8NHWC path, converted
                 // with rgb_to_nv12_kernel's integer arithmetic (elementwise.cu).  Each warp stores its own Y row; the
                 // parity-0 warp (row 2j) leaves its horizontal chroma pair sums in shared memory, the parity-1 warp (row
@@ -1095,7 +1114,7 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                 // R, G, B of the pixel pair (lanes 2i, 2i+1) as 10-bit fields: a 2x2 sum is at most 1020
                 const uint32_t hs1 = static_cast<uint32_t>(c8[0]) | (static_cast<uint32_t>(c8[1]) << 10) | (static_cast<uint32_t>(c8[2]) << 20);
                 const uint32_t hs = hs1 + __shfl_xor_sync(0xffffffffu, hs1, 1);
-                uint8_t* const frame = reinterpret_cast<uint8_t*>(E.out) + static_cast<size_t>(b.n) * (E.out_h + (E.out_h >> 1)) * E.out_w;
+                uint8_t* const frame = reinterpret_cast<uint8_t*>(E.out) + static_cast<size_t>(I.out) * (E.out_h + (E.out_h >> 1)) * E.out_w;
                 const bool st_word = valid && (lane & 3) == 0;
                 if (st_word) *reinterpret_cast<uint32_t*>(frame + static_cast<size_t>(y) * E.out_w + ax) = yw;
                 const uint32_t xchg = rec_base + kMaxSASlots * kRecWords * 4u +
@@ -1132,7 +1151,8 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
               const uint32_t lo = __shfl_sync(0xffffffffu, px, p0 & 31), hi = __shfl_sync(0xffffffffu, px, (p0 + 1) & 31);
               const uint64_t two = static_cast<uint64_t>(lo) | (static_cast<uint64_t>(hi) << 24);
               if (lane < 24) {
-                const size_t pix0 = (static_cast<size_t>(b.n) * E.out_h + y) * E.out_w + b.strip * kTileW + qd * 32;
+                const ImgAt I = ring_img(P, b.n);
+                const size_t pix0 = (static_cast<size_t>(I.out) * E.out_h + y) * E.out_w + b.strip * kTileW + qd * 32;
                 reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(E.out) + pix0 * 3)[lane] = static_cast<uint32_t>(two >> (8 * sh));
               }
             } else if (NOUT == 16 && (E.out_mode == kOutNCHWF16 || E.out_mode == kOutNCHWF32) && E.cout <= 4 &&
@@ -1140,9 +1160,10 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
               // few-channel planar output (last conv of RRDBNet / BSVD at the model boundary, optional residual on the
               // first res1_nch channels: BSVD none_minus, bsvd/model.py:436-442): one coalesced store per channel
               if (valid) {
+                const ImgAt I = ring_img(P, b.n);
                 const size_t plane = static_cast<size_t>(E.out_h) * E.out_w;
-                const size_t o0 = static_cast<size_t>(b.n) * E.cout * plane + static_cast<size_t>(y) * E.out_w + ax;
-                const uint16_t* rp = E.res1 != nullptr ? reinterpret_cast<const uint16_t*>(E.res1) + pix * E.res1_pitch + E.res1_coff : nullptr;
+                const size_t o0 = static_cast<size_t>(I.out) * E.cout * plane + static_cast<size_t>(y) * E.out_w + ax;
+                const uint16_t* rp = E.res1 != nullptr ? reinterpret_cast<const uint16_t*>(E.res1) + pix1 * E.res1_pitch + E.res1_coff : nullptr;
                 const int nres = E.res1 == nullptr ? 0 : (E.res1_nch > 0 ? E.res1_nch : E.cout);
 #pragma unroll
                 for (int c = 0; c < 4; ++c) {
@@ -1165,7 +1186,8 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
               // (factory.py:69-82).  Conv channel c*16 + a*4 + b of pixel (y, x) is out[n, c, 4y + a, 4x + b]: for one
               // (c, a) a thread owns 4 consecutive output pixels (8 bytes) and a warp 256 contiguous bytes.
               if (valid) {
-                const size_t pixi = (static_cast<size_t>(b.n) * E.out_h + y) * E.out_w + ax;
+                const ImgAt I = ring_img(P, b.n);
+                const size_t pixi = (static_cast<size_t>(I.out) * E.out_h + y) * E.out_w + ax;
                 const int OH = 4 * E.out_h, OW = 4 * E.out_w;
                 __half* const o = reinterpret_cast<__half*>(E.out);
 #pragma unroll
@@ -1181,7 +1203,7 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                     uint2 w2;
                     w2.x = *reinterpret_cast<const uint32_t*>(&lo);
                     w2.y = *reinterpret_cast<const uint32_t*>(&hi);
-                    const size_t oi = ((static_cast<size_t>(b.n) * 3 + c) * OH + (4 * y + a4)) * OW + 4 * static_cast<size_t>(ax);
+                    const size_t oi = ((static_cast<size_t>(I.out) * 3 + c) * OH + (4 * y + a4)) * OW + 4 * static_cast<size_t>(ax);
                     *reinterpret_cast<uint2*>(o + oi) = w2;
                   }
                 }
@@ -1194,7 +1216,8 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
               // shift scatter (channels [0, fold) go to frame t-1's tensor, [fold, 2 fold) to frame t+1's).  Same
               // arithmetic as epilogue_chunk, decided once per 8-channel group instead of per value.
               if (valid) {
-                const int t = E.t0 + b.n;
+                const ImgAt I = ring_img(P, b.n);
+                const int t = I.t;
                 const int cq = E.cout >> 2;
                 const bool ps2 = E.out_mode == kOutPS2NHWC;
                 const bool relu6 = E.act == kActRelu6;
@@ -1210,7 +1233,8 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                     oy = 2 * y + (ab >> 1);
                     ox = 2 * ax + (ab & 1);
                   }
-                  const size_t po = (static_cast<size_t>(b.n) * E.out_h + oy) * E.out_w + ox;
+                  const size_t po = (static_cast<size_t>(I.out) * E.out_h + oy) * E.out_w + ox;
+                  const size_t po1 = (static_cast<size_t>(I.res1) * E.out_h + oy) * E.out_w + ox;
                   float v[8];
 #pragma unroll
                   for (int i = 0; i < 8; ++i) {
@@ -1220,7 +1244,7 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                   if (E.res1 != nullptr && (E.res1_nch == 0 || oc == 0)) {
                     // (split precision: the residual tensor has a low-half twin res1_lo_off elements further on;
                     //  res1_nch > 0: only the first channels take part -- BSVD none_minus, model.py:436-442)
-                    const uint16_t* const rp = reinterpret_cast<const uint16_t*>(E.res1) + po * E.res1_pitch + E.res1_coff + oc;
+                    const uint16_t* const rp = reinterpret_cast<const uint16_t*>(E.res1) + po1 * E.res1_pitch + E.res1_coff + oc;
                     const uint4 r = *reinterpret_cast<const uint4*>(rp);
                     const uint32_t w4[4] = {r.x, r.y, r.z, r.w};
                     float rs[8];
@@ -1256,8 +1280,8 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                   int64_t delta = 0;
                   bool ok = true;
                   if (E.fold > 0) {
-                    if (oc < E.fold) { delta = E.off_prev; ok = t > 0; }
-                    else if (oc < 2 * E.fold) { delta = E.off_next; ok = t < E.t_count - 1; }
+                    if (oc < E.fold) { delta = E.off_prev * I.prev; ok = t > 0; }
+                    else if (oc < 2 * E.fold) { delta = E.off_next * I.next; ok = t < E.t_count - 1; }
                   }
                   if (ok) {
                     uint4 q4;
@@ -1278,12 +1302,13 @@ conv3x3_stream_kernel(const __grid_constant__ StreamParams P) {
                 }
               }
             } else if (valid) {
+              const ImgAt I = ring_img(P, b.n);
 #pragma unroll
               for (int c = 0; c < NOUT; c += 16) {
                 float v[16];
 #pragma unroll
                 for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(raw[c + i]);
-                epilogue_chunk(E, kModeConv3, b.n, y, ax, 0, b.chunk * NOUT + c, v);
+                epilogue_chunk(E, kModeConv3, I, y, ax, 0, b.chunk * NOUT + c, v);
               }
             }
           }

@@ -225,7 +225,7 @@ conv3x3_tcgen05_kernel(const __grid_constant__ ConvParams P) {
             float v[16];
 #pragma unroll
             for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(raw[i]);
-            epilogue_chunk(P.ep, P.mode, n, ay, ax, sub, nc * P.n_cta + cb, v);
+            epilogue_chunk(P.ep, P.mode, img_at(P.ep, n), ay, ax, sub, nc * P.n_cta + cb, v);
           }
         }
       }

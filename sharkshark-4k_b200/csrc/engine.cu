@@ -749,6 +749,7 @@ int materialize_stream(ss4k_ctx* ctx, const ConvSpec& cs, const HostTensor& W, c
   for (int kb = 0; kb < pk.nkb; ++kb) { p.a_kb[kb] = pk.src_kb[kb]; p.a_tm[kb] = pk.src_tm[kb]; p.nks[kb] = pk.nks[kb]; p.wt[kb] = pk.wt[kb]; }
   p.nwt = pk.nwt;
   p.n_in0 = cs.n0; p.n_out0 = cs.n0;   // TMA image coordinates of a step that starts inside the clip
+  p.ring_in = p.ring_out = p.ring_res1 = p.ring_res2 = -1;   // no ring wrap (BSVD streams set theirs per tensor)
   p.stride2 = pk.stride2; p.nkx = pk.nkx;
   for (int kb = 0; kb < pk.nkb; ++kb) { p.ksm[kb][0] = pk.ksm[kb][0]; p.ksm[kb][1] = pk.ksm[kb][1]; }
   p.n_img = cs.n; p.H = pk.stride2 ? cs.in_h / 2 : cs.in_h; p.W = pk.stride2 ? cs.in_w / 2 : cs.in_w;  // the output grid

@@ -77,6 +77,11 @@ def gaussian_kernel(kernel_size=3, sigma=0.5):
     return (g / g.sum()).contiguous()
 
 
+# Frames per BSVD push in temporal mode: the orchestrator hands the service jobs of up to 4 frames, so a job is one push
+# (each conv of the stream runs once over its frames instead of once per frame).
+_TEMPORAL_PUSH = 4
+
+
 class FsrcnnUpscalerService:
     LR_SHAPES = [(360, 640), (540, 960), (630, 1120), (720, 1280), (900, 1600), (1080, 1920)]  # :93-100
 
@@ -283,27 +288,30 @@ class FsrcnnUpscalerService:
         return self.upscale_multi(frames)
 
     def upscale_temporal(self, frames):
-        """upscale_single with BSVD as a temporal stream: pushes every frame into the ring-buffer engine and returns the
-        frames that left it (none for the first 16 pushes, then one per push; flush() returns the tail)."""
+        """upscale_single with BSVD as a temporal stream: pushes the job's frames into the ring-buffer engine and returns
+        the frames that left it (none for the first 16 frames, then one per frame; flush() returns the tail)."""
         lh, lw = self.lr_shape
         if self._den_stream is None:
             if self.denoise_model is None:
                 self._build_denoiser()
-            self._den_stream = self.denoise_model.stream(lh, lw)
+            self._den_stream = self.denoise_model.stream(lh, lw, max_frames=_TEMPORAL_PUSH)
+        n, ih, iw, _ = frames.shape
+        lr_before = self._area(frames, n, 3, ih, iw, lh, lw)
+        x = torch.empty(n, 4, lh, lw, dtype=torch.float32, device=self.device)
+        x[:, :3].copy_(lr_before)
+        x[:, 3].fill_(0.1 * self.denoise_rate)                                   # :262,269
+        if self.lr_prev is None:
+            x[0, 3].fill_(0.05)
+        self.lr_prev = lr_before[n - 1:n]
         done = []
-        for i in range(frames.shape[0]):
-            ih, iw, _ = frames[i].shape
-            lr_before = self._area(frames[i].unsqueeze(0), 1, 3, ih, iw, lh, lw)
-            x = torch.empty(4, lh, lw, dtype=torch.float32, device=self.device)
-            x[:3].copy_(lr_before[0])
-            x[3].fill_(0.05 if self.lr_prev is None else 0.1 * self.denoise_rate)   # :262,269
-            self.lr_prev = lr_before
-            self._lr_fifo.append(lr_before)
+        for i0 in range(0, n, _TEMPORAL_PUSH):
+            i1 = min(n, i0 + _TEMPORAL_PUSH)
+            self._lr_fifo.extend(lr_before[i:i + 1] for i in range(i0, i1))
             self.profiler.start('fsrcnn.denoise')
-            den = self._den_stream.push(x)
+            den = self._den_stream.push_frames(x[i0:i1])
             self.profiler.end('fsrcnn.denoise')
-            if den is not None:
-                done.append(self._finish_single(den, self._lr_fifo.popleft()))
+            for j in range(den.shape[0]):
+                done.append(self._finish_single(den[j:j + 1], self._lr_fifo.popleft()))
         if done:
             return torch.stack(done, dim=0)
         return self._no_frames()
